@@ -8,20 +8,26 @@ Keras-Adam lr 3e-4, batch 65 536, synthetic N(0,1) inputs with labels from a fix
 
     python bench.py [--gpus N] [--steps K] [--warmup W]            # this repo's CUDA path (weak scaling: 65 536 rows/GPU)
     python bench.py --impl reference ...                           # the reference graph's CPU twin (host cores)
-    python bench.py --config C2|C3|C4|C4p                          # the other SURVEY 8d shapes (profiles/, not the driver)
+    python bench.py --config C2|C3|C4|C4p                          # the other SURVEY 8d shapes (profiles/)
+    python bench.py --dump-outputs DIR ...                         # also write the last timed step's results to DIR
 
 Prints ONE JSON line (rank 0).
-  value / ms_per_step : device-resident throughput.  K steps per block between CUDA events (barrier + synchronize on
-                        both sides of every block), blocks repeated until the timed region is >= --min-seconds (2 s) so
-                        clocks and power are steady; the reported ms_per_step is the MEDIAN block (max over ranks).
+  value / ms_per_step : device-resident throughput.  Exactly K steps between two CUDA events (barrier + synchronize on
+                        both sides) after W untimed warm-up steps; ms_per_step is their mean (max over ranks).
   strong              : the same metric with the 65 536-row GLOBAL batch split over the N GPUs (SURVEY 8d "the metric as
                         stated"), measured in the same run (for N = 1 it equals value).
   e2e                 : the same step through the public API (model.train_on_batch) from pinned HOST buffers with the
-                        H2D copy and the D2H read of the metrics inside the timed region.
+                        H2D copy and the D2H read of the metrics inside the timed region (another K steps).
   roofline            : the dominant kernel's algorithmic FLOP/s (SURVEY 8d MAC counts) over its CUDA-event duration,
                         against the measured dense bf16/fp16 tensor peak -- burst or sustained chosen from the SM clock
                         sampled during the timed region.
 See DESIGN.md section "Measurement".
+
+--dump-outputs DIR writes, after the device-resident timed steps and before anything else trains the model further, what
+a caller of the timed path (model.train_on_batch) receives from its last step: the metrics (loss.npy, accuracy.npy,
+kl_per_feature.npy, float64) and the updated weights (weights.npy, the flat float32 parameter vector).  Inputs, initial
+weights and noise are seeded, so the same arguments give the same inputs on every run and two builds can be compared
+output for output.
 """
 import argparse
 import glob
@@ -281,6 +287,17 @@ def workload_config(cfg, name, n_gpus=None, precision=None, per_gpu=None):
                   "activations/gradients/partials per 65536 rows), evicting the 16 rotating input batches between their uses"}
 
 
+def dump_outputs(out_dir, metrics, weights, F):
+    """What train_on_batch hands its caller for one step: the metrics dict and the model's updated weights."""
+    os.makedirs(out_dir, exist_ok=True)
+    arrays = {"loss": np.array([metrics["loss"]], dtype=np.float64),
+              "accuracy": np.array([metrics["accuracy"]], dtype=np.float64),
+              "kl_per_feature": np.array([metrics[f"KL{i}"] for i in range(F)], dtype=np.float64),
+              "weights": np.asarray(weights, dtype=np.float32)}
+    for name, a in arrays.items():
+        np.save(os.path.join(out_dir, name + ".npy"), a)
+
+
 JSON_OUT = None
 
 
@@ -310,11 +327,12 @@ def main():
                     help="fp16 = fused tcgen05 kernels on fp16 operands (default, the headline); bf16 likewise; "
                          "tf32 = kind::tf32 GEMMs on fp32 storage; fp32 = exact CUDA-core parity path")
     ap.add_argument("--config", default="C0", choices=sorted(CONFIGS))
-    ap.add_argument("--min-seconds", type=float, default=2.0, help="lower bound on the device-timed region")
+    ap.add_argument("--dump-outputs", metavar="DIR",
+                    help="write the last timed step's metrics and updated weights to DIR/<name>.npy")
     ap.add_argument("--no-cpu-baseline", action="store_true")
     ap.add_argument("--no-strong", action="store_true")
     ap.add_argument("--scaling", default="weak", choices=["weak", "strong"],
-                    help="what `value` reports -- weak (default, the driver's contract): the config batch per GPU; strong: the "
+                    help="what `value` reports -- weak (default): the config batch per GPU; strong: the "
                          "global batch split over the GPUs.  The other one is always reported under its own key.")
     args = ap.parse_args()
     cfg = CONFIGS[args.config]
@@ -322,6 +340,8 @@ def main():
     world = int(os.environ.get("WORLD_SIZE", "1"))
     local_rank = int(os.environ.get("LOCAL_RANK", "0"))
     if args.impl == "reference":
+        if args.dump_outputs:
+            ap.error("--dump-outputs writes what the CUDA path computed; it does not apply to --impl reference")
         run_reference(args, rank, cfg)
         return
     args.warmup = max(args.warmup, 3)
@@ -358,46 +378,43 @@ def main():
         dist.all_reduce(t, op=dist.ReduceOp.MAX)
         return float(t.item())
 
-    def timed_blocks(step_fn, steps, min_seconds, max_blocks=4000):
-        """Blocks of exactly `steps` steps, each between CUDA events with barrier + synchronize on both sides; repeated
-        until the device-timed total reaches min_seconds.  Returns (median block ms [max over ranks], total s, blocks)."""
+    def timed(step_fn, steps):
+        """Exactly `steps` steps between CUDA events with barrier + synchronize on both sides.
+        Returns (ms per step [max over ranks], total s)."""
         ev0, ev1 = torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True)
-        times, total, it = [], 0.0, 0
-        while True:
-            barrier()
-            ev0.record()
-            for _ in range(steps):
-                step_fn(it)
-                it += 1
-            ev1.record()
-            barrier()
-            ms = max_over_ranks(ev0.elapsed_time(ev1))
-            times.append(ms)
-            total += ms * 1e-3
-            if total >= min_seconds or len(times) >= max_blocks:
-                break
-        return float(np.median(times)), total, len(times)
+        barrier()
+        ev0.record()
+        for i in range(steps):
+            step_fn(i)
+        ev1.record()
+        barrier()
+        ms = max_over_ranks(ev0.elapsed_time(ev1))
+        return ms / steps, ms * 1e-3
 
-    def measure(PB, min_seconds, with_e2e):
+    def measure(PB, with_e2e, dump_dir=None):
         """Device-resident and (optionally) end-to-end throughput at PB rows per GPU."""
         xs_h, ys_h = synth_batches(cfg, rank, N_DISTINCT_BATCHES, PB, pinned=True)
         xs_d = [x.cuda(non_blocking=True) for x in xs_h]
         ys_d = [y.cuda(non_blocking=True) for y in ys_h]
         torch.cuda.synchronize()
 
+        last_result = [None]
+
         def device_step(i):       # public API, device-resident batch, no host read inside the step
-            model.train_on_batch(xs_d[i % N_DISTINCT_BATCHES], ys_d[i % N_DISTINCT_BATCHES], sync=False)
+            last_result[0] = model.train_on_batch(xs_d[i % N_DISTINCT_BATCHES], ys_d[i % N_DISTINCT_BATCHES], sync=False)
 
         for i in range(args.warmup):
             device_step(i)
         barrier()
         count = lambda: int(lib.dib_launch_count()) + int(getattr(model, "_replayed_launches", 0))   # eager + graph-replayed kernels
         launches0 = count()
-        blk_ms, total_s, nblk = timed_blocks(device_step, args.steps, min_seconds)
+        ms_step, total_s = timed(device_step, args.steps)
         launches = count() - launches0
-        res = {"ms_per_step": blk_ms / args.steps, "timed_region_s": total_s, "blocks": nblk, "launches": launches,
-               "launches_per_step": launches / (nblk * args.steps), "xs_d": xs_d, "ys_d": ys_d}
+        res = {"ms_per_step": ms_step, "timed_region_s": total_s, "launches": launches,
+               "launches_per_step": launches / args.steps, "xs_d": xs_d, "ys_d": ys_d}
         res["value"] = PB * world / (res["ms_per_step"] * 1e-3)
+        if dump_dir is not None:
+            dump_outputs(dump_dir, last_result[0].get(), model.get_flat_weights(), F)
         if with_e2e:
             for i in range(3):
                 model.train_on_batch(xs_h[i], ys_h[i], sync=False).get()
@@ -410,12 +427,11 @@ def main():
                 if len(pend) > 4:
                     last.update(pend.pop(0).get())       # the host reads every step's result, a few steps behind the device
 
-            blk, tot, nb = timed_blocks(e2e_step, args.steps, min(min_seconds, 1.0))
+            e2e_ms, tot = timed(e2e_step, args.steps)
             for p in pend:
                 last.update(p.get())
-            e2e_ms = blk / args.steps
             res["e2e"] = {"value": PB * world / (e2e_ms * 1e-3), "unit": "samples/s", "ms_per_step": e2e_ms,
-                          "timed_region_s": tot, "blocks": nb,
+                          "timed_region_s": tot,
                           "h2d_bytes_per_step": int(xs_h[0].numel() * 4 + ys_h[0].numel() * 4),
                           "d2h_bytes_per_step": int((F + 3) * 4),
                           "api": "DistributedIBNet.train_on_batch(host x, host y, sync=False).get() -> metrics dict "
@@ -428,10 +444,10 @@ def main():
     PB_weak = BATCH
     PB_strong = max(BATCH // world, 1)
     primary_PB = PB_weak if args.scaling == "weak" else PB_strong
-    prim = measure(primary_PB, args.min_seconds, with_e2e=True)
+    prim = measure(primary_PB, with_e2e=True, dump_dir=args.dump_outputs if rank == 0 else None)
     other = None
     if world > 1 and not args.no_strong:
-        other = measure(PB_strong if args.scaling == "weak" else PB_weak, min(args.min_seconds, 1.0), with_e2e=False)
+        other = measure(PB_strong if args.scaling == "weak" else PB_weak, with_e2e=False)
     clocks = sampler.stop() if sampler else None
     weak, strong = (prim, other) if args.scaling == "weak" else (other, prim)
     if world == 1:
@@ -492,14 +508,15 @@ def main():
     if rank == 0:
         pack = lambda r, pb: None if r is None else {"value": r["value"], "unit": "samples/s", "ms_per_step": r["ms_per_step"],
                                                      "per_gpu_batch": pb, "global_batch": pb * world,
-                                                     "timed_region_s": r["timed_region_s"], "blocks": r["blocks"]}
+                                                     "timed_region_s": r["timed_region_s"]}
         line = {
             "metric": METRIC, "value": prim["value"], "unit": "samples/s", "n_gpus": world, "steps": args.steps,
             "warmup": args.warmup, "ms_per_step": ms_per_step, "higher_is_better": True, "scaling": args.scaling,
             "vs_baseline": None, "dtype": DTYPE_LABEL[args.precision],
             "data": "synthetic", "config": workload_config(cfg, args.config, world, args.precision, PB),
-            "timed_region_s": prim["timed_region_s"], "blocks": prim["blocks"],
-            "timing": f"median of {prim['blocks']} blocks of {args.steps} steps (CUDA events, barrier+sync around each block, max over ranks)",
+            "timed_region_s": prim["timed_region_s"],
+            "timing": f"mean of {args.steps} steps after {args.warmup} warm-up steps (CUDA events, barrier+sync around "
+                      f"the timed region, max over ranks)",
             "weak": pack(weak, PB_weak), "strong": pack(strong, PB_strong),
             "clocks": clocks, "e2e": prim.get("e2e"),
             "gpu_launches": prim["launches"], "launches_per_step": prim["launches_per_step"],

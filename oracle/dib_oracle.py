@@ -18,6 +18,8 @@ the product path (dib_b200) never does.
 """
 from __future__ import annotations
 
+import ast
+import hashlib
 import math
 from dataclasses import dataclass, field
 from typing import Callable, List, Optional, Sequence
@@ -153,6 +155,29 @@ def glorot_uniform_params(cfg: DIBConfig, rng: np.random.Generator, dtype=np.flo
         else:
             out.append(np.zeros(s, dtype=dtype))
     return np.concatenate(out)
+
+
+def golden_case_params(cfg: DIBConfig, seed: int):
+    """Weights of a tests/golden/ref_forward_*.npz case: glorot-uniform kernels and N(0, 0.05^2) biases (non-zero, so
+    that bias handling is pinned) drawn from default_rng(seed).  Returns (weights, rng); the case's inputs come next."""
+    rng = np.random.default_rng(seed)
+    flat = glorot_uniform_params(cfg, rng, dtype=np.float32)
+    flat = flat + (rng.standard_normal(flat.size) * 0.05).astype(np.float32) * (flat == 0)
+    return flat, rng
+
+
+def load_forward_golden(path):
+    """(cfg, arrays) of a tests/golden/ref_forward_*.npz case.  The weights are not stored (C0's alone are 2.4 MB of
+    incompressible floats): they are regenerated from the stored seed and checked against the SHA-256 of the weights
+    the reference computed the case with, so a change in numpy's random streams fails loudly instead of comparing
+    against the wrong model."""
+    z = dict(np.load(path))
+    cfg = DIBConfig(**ast.literal_eval(str(z["cfg"])))
+    params, _ = golden_case_params(cfg, int(z["seed"]))
+    if hashlib.sha256(params.tobytes()).hexdigest() != str(z["params_sha256"]):
+        raise RuntimeError(f"{path}: the weights regenerated from seed {int(z['seed'])} are not the golden's")
+    z["params"] = params
+    return cfg, z
 
 
 def unflatten(cfg: DIBConfig, flat: np.ndarray):

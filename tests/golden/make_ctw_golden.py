@@ -1,6 +1,7 @@
-"""Generates tests/golden/ref_ctw.npz from the REFERENCE'S OWN native code: chaos/cppctw.cpp compiled where it lies
-(oracle/Makefile -> oracle/_ref/libctw_ref.so).  Run in the build container (needs /root/reference):
-    make -C oracle && python tests/golden/make_ctw_golden.py"""
+"""Generates tests/golden/ref_ctw.npz and ref_ctw_sweeps.npz from the REFERENCE'S OWN native code: chaos/cppctw.cpp
+compiled where it lies in a checkout of the reference (oracle/Makefile -> oracle/_ref/libctw_ref.so):
+    make -C oracle REF=<reference checkout> && python tests/golden/make_ctw_golden.py
+ref_ctw_sweeps.npz holds the reference's entropy for each sequence of the seeded sweeps in tests/test_ctw.py."""
 import os
 import sys
 
@@ -9,6 +10,7 @@ import numpy as np
 HERE = os.path.dirname(os.path.abspath(__file__))
 sys.path.insert(0, os.path.join(HERE, "..", ".."))
 from oracle import ctw_oracle  # noqa: E402
+from tests.test_ctw import fresh_sequences, small_sequences  # noqa: E402
 
 
 def sequences():
@@ -43,6 +45,10 @@ def main():
         rec[name + "_H"] = np.float64(ctw_oracle.reference_estimate_entropy(seq, A))
         print(f"{name:>20s}  A={A:<3d} n={len(seq):<6d} H={rec[name + '_H']!r}")
     np.savez_compressed(os.path.join(HERE, "ref_ctw.npz"), **rec)
+    sweeps = {key: np.array([ctw_oracle.reference_estimate_entropy(seq, A) for seq, A in cases()], dtype=np.float64)
+              for key, cases in (("fresh_H", fresh_sequences), ("small_H", small_sequences))}
+    np.savez_compressed(os.path.join(HERE, "ref_ctw_sweeps.npz"), **sweeps)
+    print({k: len(v) for k, v in sweeps.items()})
 
 
 if __name__ == "__main__":

@@ -14,6 +14,7 @@ Run here (needs /root/reference; never run on the GPU box):
     python tests/golden/make_golden.py
 Writes tests/golden/*.npz, which are committed.
 """
+import hashlib
 import os
 import sys
 import types
@@ -222,10 +223,7 @@ def run_case(models, name, cfg_kwargs, B, beta, seed):
     sys.path.insert(0, os.path.join(HERE, "..", ".."))
     from oracle import dib_oracle as O
     cfg = O.DIBConfig(**cfg_kwargs)
-    rng = np.random.default_rng(seed)
-    flat = O.glorot_uniform_params(cfg, rng, dtype=np.float32)
-    # give biases non-zero values so that bias handling is actually pinned
-    flat = flat + (rng.standard_normal(flat.size) * 0.05).astype(np.float32) * (flat == 0)
+    flat, rng = O.golden_case_params(cfg, seed)
     D = int(np.sum(cfg.feature_dimensionalities))
     x = rng.standard_normal((B, D)).astype(np.float32)
     eps = rng.standard_normal((B, cfg.number_features, cfg.feature_embedding_dimension)).astype(np.float32)
@@ -244,7 +242,9 @@ def run_case(models, name, cfg_kwargs, B, beta, seed):
     assert not EPS.q
     kls = np.array([model.metrics_log[f"KL{i}"] for i in range(cfg.number_features)])
     enc_out = [model.feature_encoders[i](_split(x.astype(DT), list(fd))[i]) for i in range(len(fd))]
-    out = dict(params=flat, x=x, eps=eps, beta=np.float32(beta), pred=np.asarray(pred),
+    # the weights are regenerated from the seed when loaded (oracle.dib_oracle.load_forward_golden): only their digest is kept
+    out = dict(seed=np.int64(seed), params_sha256=np.array(hashlib.sha256(flat.tobytes()).hexdigest()),
+               x=x, eps=eps, beta=np.float32(beta), pred=np.asarray(pred),
                kl=kls, ib_loss=np.asarray(model.losses[0]), beta_metric=model.metrics_log["beta"],
                cfg=np.array(repr(cfg_kwargs)))
     for i, o in enumerate(enc_out):

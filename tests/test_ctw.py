@@ -1,6 +1,6 @@
 """Next row f4: the CTW entropy-rate estimator.  Host code (no GPU): the C-ABI functions are compared BIT-EXACTLY with
  (a) goldens produced by the reference's own chaos/cppctw.cpp (tests/golden/ref_ctw.npz, make_ctw_golden.py),
- (b) the reference's build itself when oracle/_ref/libctw_ref.so is present (oracle/Makefile),
+ (b) the reference build's results on seeded sweeps of fresh sequences (tests/golden/ref_ctw_sweeps.npz, same script),
  (c) the Python restatement oracle/ctw_oracle.py on small sequences."""
 import os
 
@@ -39,16 +39,48 @@ def test_library_matches_reference_goldens_bit_exactly(ctw, golden_dir):
         np.testing.assert_array_equal(got, [c[3] for c in group])
 
 
-@pytest.mark.skipif(not ctw_oracle.reference_available(), reason="oracle/_ref/libctw_ref.so not built (make -C oracle)")
-def test_library_matches_reference_build_on_fresh_sequences(ctw):
+def fresh_sequences():
+    """(sequence, alphabet size) pairs of the fresh-sequence comparison; make_ctw_golden.py stores the reference's results."""
     rng = np.random.default_rng(123)
-    for n, A in ((0, 2), (1, 3), (33, 2), (1000, 3), (6000, 4), (3000, 27)):
-        if n == 0:
-            assert np.isnan(ctw.estimate_entropy([], A))
-            continue
+    out = []
+    for n, A in ((1, 3), (33, 2), (1000, 3), (6000, 4), (3000, 27)):
         seq = rng.integers(0, A, n)
         seq[n // 3: n // 3 + min(n // 4, 900)] = seq[0]                       # a long run: deep tails, depth > 512
-        assert ctw.estimate_entropy(seq, A) == ctw_oracle.reference_estimate_entropy(seq, A), (n, A)
+        out.append((seq, A))
+    return out
+
+
+def small_sequences():
+    """(sequence, alphabet size) pairs of the small-sequence sweep: short sequences over small alphabets, incl. long runs
+    and periodic pieces that exercise the lazy tail extension; make_ctw_golden.py stores the reference's results."""
+    rng = np.random.default_rng(2024)
+    out = []
+    for trial in range(300):
+        A = int(rng.integers(1, 6))
+        n = int(rng.integers(1, 90))
+        kind = trial % 3
+        if kind == 0:
+            seq = rng.integers(0, A, n)
+        elif kind == 1:                                                       # runs
+            seq = np.repeat(rng.integers(0, A, max(n // 7, 1)), 7)[:n]
+        else:                                                                 # periodic with a defect
+            seq = np.tile(rng.integers(0, A, int(rng.integers(1, 5))), n)[:n]
+            seq[int(rng.integers(0, n))] = int(rng.integers(0, A))
+        out.append((seq, A))
+    return out
+
+
+def _sweep_goldens(golden_dir, key, cases):
+    want = np.load(os.path.join(golden_dir, "ref_ctw_sweeps.npz"))[key]
+    assert len(want) == len(cases)
+    return want
+
+
+def test_library_matches_reference_build_on_fresh_sequences(ctw, golden_dir):
+    assert np.isnan(ctw.estimate_entropy([], 2))
+    cases = fresh_sequences()
+    for (seq, A), H in zip(cases, _sweep_goldens(golden_dir, "fresh_H", cases)):
+        assert ctw.estimate_entropy(seq, A) == H, (len(seq), A)
 
 
 def test_edge_cases_and_errors(ctw):
@@ -76,22 +108,10 @@ def test_entropy_rate_properties(ctw):
     assert abs(ctw.estimate_entropy(markov, 2) - (-(0.05 * np.log2(0.05) + 0.95 * np.log2(0.95)))) < 0.02
 
 
-def test_random_small_sequences_against_python_restatement(ctw):
-    """hypothesis-style sweep (seeded): many short sequences over small alphabets, incl. long runs and periodic pieces
-    that exercise the lazy tail extension; library == Python restatement == (when built) the reference, bit for bit."""
-    rng = np.random.default_rng(2024)
-    for trial in range(300):
-        A = int(rng.integers(1, 6))
-        n = int(rng.integers(1, 90))
-        kind = trial % 3
-        if kind == 0:
-            seq = rng.integers(0, A, n)
-        elif kind == 1:                                                       # runs
-            seq = np.repeat(rng.integers(0, A, max(n // 7, 1)), 7)[:n]
-        else:                                                                 # periodic with a defect
-            seq = np.tile(rng.integers(0, A, int(rng.integers(1, 5))), n)[:n]
-            seq[int(rng.integers(0, n))] = int(rng.integers(0, A))
+def test_random_small_sequences_against_python_restatement(ctw, golden_dir):
+    """hypothesis-style sweep (seeded): library == Python restatement == the reference, bit for bit."""
+    cases = small_sequences()
+    for trial, ((seq, A), H) in enumerate(zip(cases, _sweep_goldens(golden_dir, "small_H", cases))):
         got = ctw.estimate_entropy(seq, A)
         assert got == ctw_oracle.estimate_entropy(seq, A), (trial, A, seq.tolist())
-        if ctw_oracle.reference_available():
-            assert got == ctw_oracle.reference_estimate_entropy(seq, A), (trial, A, seq.tolist())
+        assert got == H, (trial, A, seq.tolist())

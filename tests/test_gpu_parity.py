@@ -3,7 +3,6 @@
  (b) the float64 CPU oracle on the same seeded inputs,
  (c) size-independent properties at the BASELINE batch (65 536): shard additivity, determinism.
 Tolerances are fp32-vs-float64 reduction-order tolerances and are written next to each check."""
-import ast
 import os
 
 import numpy as np
@@ -33,8 +32,7 @@ def build_model(cfg, precision="fp32", loss="bce_logits", lr=1e-3, seed=0):
 
 
 def load_case(golden_dir, name):
-    z = np.load(os.path.join(golden_dir, f"ref_forward_{name}.npz"))
-    return O.DIBConfig(**ast.literal_eval(str(z["cfg"]))), z
+    return O.load_forward_golden(os.path.join(golden_dir, f"ref_forward_{name}.npz"))
 
 
 def make_labels(rng, loss, B, out):

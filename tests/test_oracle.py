@@ -1,7 +1,6 @@
 """CPU: the oracle against (i) golden vectors produced by the reference's own code (tests/golden/
 make_golden.py), (ii) the closed-form known answers of SURVEY.md section 4, (iii) itself (finite differences,
 torch-autograd twin, data-parallel shard additivity)."""
-import ast
 import os
 
 import numpy as np
@@ -14,9 +13,7 @@ CASES = ["c0_small", "pendulum_like", "radial_like", "odd_shapes"]
 
 
 def load_case(golden_dir, name):
-    z = np.load(os.path.join(golden_dir, f"ref_forward_{name}.npz"))
-    cfg = O.DIBConfig(**ast.literal_eval(str(z["cfg"])))
-    return cfg, z
+    return O.load_forward_golden(os.path.join(golden_dir, f"ref_forward_{name}.npz"))
 
 
 @pytest.mark.parametrize("name", CASES)
