@@ -77,6 +77,9 @@ SIGNATURES = {
     "dib_scaled_similarity": (c_int32, [c_int32, c_void_p, c_int64, c_void_p, c_int64, c_int32, c_float, c_void_p, c_void_p]),
     "dib_infonce_head": (c_int32, [c_int32, c_void_p, c_void_p, c_int64, c_int32, c_float, c_void_p, c_void_p, c_void_p,
                                    c_void_p, c_void_p]),
+    "dib_infonce_head_tc_scratch_bytes": (c_int64, [c_int64, c_int32]),
+    "dib_infonce_head_tc": (c_int32, [c_int32, c_void_p, c_void_p, c_int64, c_int32, c_float, c_void_p, c_void_p, c_void_p,
+                                      c_void_p, c_void_p]),
     "dib_ctw_estimate_entropy": (c_int32, [c_void_p, c_int64, c_int32, c_void_p]),
     "dib_ctw_estimate_entropy_batch": (c_int32, [c_void_p, c_void_p, c_int32, c_int32, c_int32, c_void_p]),
     "dib_ctw_last_error": (c_char_p, []),

@@ -1211,6 +1211,24 @@ int dib_infonce_head(int32_t kind, const float* e1, const float* e2, int64_t n, 
   return 0;
 }
 
+int64_t dib_infonce_head_tc_scratch_bytes(int64_t n, int32_t d) {
+  if (n < 1 || n > (1 << 26) || d < 1 || d > 256) return -1;
+  return (int64_t)dib_infonce_head_tc_scratch(n, d);
+}
+
+int dib_infonce_head_tc(int32_t kind, const float* e1, const float* e2, int64_t n, int32_t d, float temperature, void* scratch,
+                        float* out_loss, float* d_e1, float* d_e2, void* stream) {
+  if ((kind != 0 && kind != 1 && kind != 4) || n < 1 || n > (1 << 26) || d < 1 || d > 256 || !(temperature > 0.f) || !e1 ||
+      !e2 || !scratch || !out_loss)
+    return fail("dib_infonce_head_tc: bad arguments (kind l2sq/l2/cosine, 1 <= n <= 2^26, 1 <= d <= 256, temperature > 0)");
+  if (reinterpret_cast<uintptr_t>(scratch) % 128)
+    return fail("dib_infonce_head_tc: scratch must be 128-byte aligned");
+  if (!dib_infonce_head_tc_available()) return fail("dib_infonce_head_tc: cuTensorMapEncodeTiled is not available");
+  DIB_CUDA_OK(dib_launch_infonce_head_tc(kind, e1, e2, n, d, temperature, scratch, out_loss, d_e1, d_e2,
+                                         static_cast<cudaStream_t>(stream)));
+  return 0;
+}
+
 int dib_compression_matrices(dib_model* h, const float* params, const float* x, int64_t n_total, const int32_t* row_index,
                              int64_t n, float* out_mu_logvar, float* out_dist, float* out_compression, void* workspace,
                              void* stream) {

@@ -1270,20 +1270,6 @@ __global__ void dib_enc_pack_weights_kernel(const float* __restrict__ params, co
   out[(long long)f * kPackElems + idx] = h;
 }
 
-typedef CUresult (*EncodeTiledFn)(CUtensorMap*, CUtensorMapDataType, cuuint32_t, void*, const cuuint64_t*,
-                                  const cuuint64_t*, const cuuint32_t*, const cuuint32_t*, CUtensorMapInterleave,
-                                  CUtensorMapSwizzle, CUtensorMapL2promotion, CUtensorMapFloatOOBfill);
-EncodeTiledFn encode_fn2() {
-  static EncodeTiledFn fn = nullptr;
-  if (!fn) {
-    void* p = nullptr;
-    cudaDriverEntryPointQueryResult q;
-    if (cudaGetDriverEntryPoint("cuTensorMapEncodeTiled", &p, cudaEnableDefault, &q) == cudaSuccess &&
-        q == cudaDriverEntryPointSuccess)
-      fn = reinterpret_cast<EncodeTiledFn>(p);
-  }
-  return fn;
-}
 
 // [rows x cols] 16-bit matrix per feature -> 3D map (col, row, feature), box 64 cols x rows x 1, SWIZZLE_128B
 bool make_wmap(CUtensorMap* m, const uint16_t* base, int cols, int rows, int nfeat, bool bf16) {
@@ -1291,7 +1277,7 @@ bool make_wmap(CUtensorMap* m, const uint16_t* base, int cols, int rows, int nfe
   cuuint64_t strides[2] = {(cuuint64_t)cols * 2, (cuuint64_t)kPackElems * 2};
   cuuint32_t box[3] = {64, (cuuint32_t)rows, 1};
   cuuint32_t es[3] = {1, 1, 1};
-  return encode_fn2()(m, bf16 ? CU_TENSOR_MAP_DATA_TYPE_BFLOAT16 : CU_TENSOR_MAP_DATA_TYPE_FLOAT16, 3,
+  return tensor_map_encode_fn()(m, bf16 ? CU_TENSOR_MAP_DATA_TYPE_BFLOAT16 : CU_TENSOR_MAP_DATA_TYPE_FLOAT16, 3,
                       const_cast<uint16_t*>(base), dims, strides, box, es, CU_TENSOR_MAP_INTERLEAVE_NONE,
                       CU_TENSOR_MAP_SWIZZLE_128B, CU_TENSOR_MAP_L2_PROMOTION_L2_256B,
                       CU_TENSOR_MAP_FLOAT_OOB_FILL_NONE) == CUDA_SUCCESS;
@@ -1314,7 +1300,7 @@ bool make_a0_maps(WeightMaps* m, const void* a0g, long long n, int F, bool bf16)
   cuuint32_t box[3] = {8, (cuuint32_t)TM, 1};
   cuuint32_t es[3] = {1, 1, 1};
   const CUtensorMapDataType dt = bf16 ? CU_TENSOR_MAP_DATA_TYPE_BFLOAT16 : CU_TENSOR_MAP_DATA_TYPE_FLOAT16;
-  if (encode_fn2()(&m->a0lo, dt, 3, const_cast<void*>(a0g), dims, strides, box, es, CU_TENSOR_MAP_INTERLEAVE_NONE,
+  if (tensor_map_encode_fn()(&m->a0lo, dt, 3, const_cast<void*>(a0g), dims, strides, box, es, CU_TENSOR_MAP_INTERLEAVE_NONE,
                    CU_TENSOR_MAP_SWIZZLE_NONE, CU_TENSOR_MAP_L2_PROMOTION_L2_256B, CU_TENSOR_MAP_FLOAT_OOB_FILL_NONE) != CUDA_SUCCESS)
     return false;
   m->a0hi = m->a0lo;
@@ -1367,7 +1353,7 @@ cudaError_t dib_enc_fused_pack(const DibEncFusedDesc& d, const float* params, vo
 }
 
 cudaError_t dib_enc_fused_forward(const DibEncFusedDesc& d, const DibEncFusedIO& io, cudaStream_t st) {
-  if (!encode_fn2()) return cudaErrorNotSupported;
+  if (!tensor_map_encode_fn()) return cudaErrorNotSupported;
   WeightMaps m;
   if (!make_all_maps(&m, io.packed, d.F, d.bf16)) return cudaErrorInvalidValue;
   EncFusedParams P;
@@ -1382,7 +1368,7 @@ cudaError_t dib_enc_fused_forward(const DibEncFusedDesc& d, const DibEncFusedIO&
 
 cudaError_t dib_enc_fused_backward(const DibEncFusedDesc& d, const DibEncFusedIO& io, const DibEncFusedBwdIO& b,
                                    cudaStream_t st) {
-  if (!encode_fn2()) return cudaErrorNotSupported;
+  if (!tensor_map_encode_fn()) return cudaErrorNotSupported;
   WeightMaps m;
   if (!make_all_maps(&m, io.packed, d.F, d.bf16)) return cudaErrorInvalidValue;
   EncFusedBwdParams Q;

@@ -217,21 +217,6 @@ dib_gemm_tc_kernel(const __grid_constant__ CUtensorMap mapA, const __grid_consta
 }
 
 // ------------------------------------------------------------------------------------------------ host side
-typedef CUresult (*EncodeTiledFn)(CUtensorMap*, CUtensorMapDataType, cuuint32_t, void*, const cuuint64_t*,
-                                  const cuuint64_t*, const cuuint32_t*, const cuuint32_t*, CUtensorMapInterleave,
-                                  CUtensorMapSwizzle, CUtensorMapL2promotion, CUtensorMapFloatOOBfill);
-
-EncodeTiledFn encode_fn() {
-  static EncodeTiledFn fn = nullptr;
-  if (!fn) {
-    void* p = nullptr;
-    cudaDriverEntryPointQueryResult q;
-    if (cudaGetDriverEntryPoint("cuTensorMapEncodeTiled", &p, cudaEnableDefault, &q) == cudaSuccess &&
-        q == cudaDriverEntryPointSuccess)
-      fn = reinterpret_cast<EncodeTiledFn>(p);
-  }
-  return fn;
-}
 
 // K-major operand: matrix [rows x ld] fp32, feature stride fs floats -> 3D map (col, row, feature), box 32 x brows x 1
 bool make_map_kmajor(CUtensorMap* m, const float* base, long long cols, long long rows, long long ld, long long fs,
@@ -240,7 +225,7 @@ bool make_map_kmajor(CUtensorMap* m, const float* base, long long cols, long lon
   cuuint64_t strides[2] = {(cuuint64_t)ld * 4, (cuuint64_t)(nfeat > 1 ? fs : ld * rows) * 4};
   cuuint32_t box[3] = {32, (cuuint32_t)box_rows, 1};
   cuuint32_t es[3] = {1, 1, 1};
-  return encode_fn()(m, CU_TENSOR_MAP_DATA_TYPE_FLOAT32, 3, const_cast<float*>(base), dims, strides, box, es,
+  return tensor_map_encode_fn()(m, CU_TENSOR_MAP_DATA_TYPE_FLOAT32, 3, const_cast<float*>(base), dims, strides, box, es,
                      CU_TENSOR_MAP_INTERLEAVE_NONE, CU_TENSOR_MAP_SWIZZLE_128B, CU_TENSOR_MAP_L2_PROMOTION_L2_256B,
                      CU_TENSOR_MAP_FLOAT_OOB_FILL_NONE) == CUDA_SUCCESS;
 }
@@ -254,7 +239,7 @@ bool make_map_mnmajor(CUtensorMap* m, const float* base, long long cols, long lo
   cuuint64_t strides[3] = {(cuuint64_t)ld * 4, 128, (cuuint64_t)(nfeat > 1 ? fs : ld * krows) * 4};
   cuuint32_t box[4] = {32, (cuuint32_t)kBK, (cuuint32_t)npanels, 1};
   cuuint32_t es[4] = {1, 1, 1, 1};
-  return encode_fn()(m, CU_TENSOR_MAP_DATA_TYPE_FLOAT32, 4, const_cast<float*>(base), dims, strides, box, es,
+  return tensor_map_encode_fn()(m, CU_TENSOR_MAP_DATA_TYPE_FLOAT32, 4, const_cast<float*>(base), dims, strides, box, es,
                      CU_TENSOR_MAP_INTERLEAVE_NONE, CU_TENSOR_MAP_SWIZZLE_128B_ATOM_32B, CU_TENSOR_MAP_L2_PROMOTION_L2_256B,
                      CU_TENSOR_MAP_FLOAT_OOB_FILL_NONE) == CUDA_SUCCESS;
 }
@@ -286,7 +271,7 @@ cudaError_t launch_tc(const DibGemmLaunch& L, const CUtensorMap& mapA, const CUt
 // Can this group of problems (host copies) run on the tensor-core kernel?  See the operand-major table above.
 bool dib_gemm_tc_eligible(int mode, const DibGemmProblem* hp, int nprob, const float* params_base_hint) {
   (void)params_base_hint;
-  if (!encode_fn() || nprob < 1) return false;
+  if (!tensor_map_encode_fn() || nprob < 1) return false;
   const DibGemmProblem& p0 = hp[0];
   const long long sa = nprob > 1 ? hp[1].a_off - hp[0].a_off : 0, sb = nprob > 1 ? hp[1].b_off - hp[0].b_off : 0;
   for (int i = 0; i < nprob; ++i) {

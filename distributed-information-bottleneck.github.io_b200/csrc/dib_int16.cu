@@ -1333,25 +1333,12 @@ __global__ void dib_f32_to_16_kernel(const float* __restrict__ src, uint16_t* __
   }
 }
 
-typedef CUresult (*EncodeTiledFn)(CUtensorMap*, CUtensorMapDataType, cuuint32_t, void*, const cuuint64_t*,
-                                  const cuuint64_t*, const cuuint32_t*, const cuuint32_t*, CUtensorMapInterleave,
-                                  CUtensorMapSwizzle, CUtensorMapL2promotion, CUtensorMapFloatOOBfill);
-EncodeTiledFn encode_fn3() {
-  static EncodeTiledFn fn = nullptr;
-  if (!fn) {
-    void* p = nullptr;
-    cudaDriverEntryPointQueryResult q;
-    if (cudaGetDriverEntryPoint("cuTensorMapEncodeTiled", &p, cudaEnableDefault, &q) == cudaSuccess && q == cudaDriverEntryPointSuccess)
-      fn = reinterpret_cast<EncodeTiledFn>(p);
-  }
-  return fn;
-}
 // K-major: [rows x ld] fp16, box 64 cols x brows
 bool map_k(CUtensorMap* m, const void* base, long long cols, long long rows, long long ld, int brows) {
   cuuint64_t dims[2] = {(cuuint64_t)cols, (cuuint64_t)rows};
   cuuint64_t strides[1] = {(cuuint64_t)ld * 2};
   cuuint32_t box[2] = {64, (cuuint32_t)brows}, es[2] = {1, 1};
-  return encode_fn3()(m, CU_TENSOR_MAP_DATA_TYPE_FLOAT16, 2, const_cast<void*>(base), dims, strides, box, es,
+  return tensor_map_encode_fn()(m, CU_TENSOR_MAP_DATA_TYPE_FLOAT16, 2, const_cast<void*>(base), dims, strides, box, es,
                       CU_TENSOR_MAP_INTERLEAVE_NONE, CU_TENSOR_MAP_SWIZZLE_128B, CU_TENSOR_MAP_L2_PROMOTION_L2_256B,
                       CU_TENSOR_MAP_FLOAT_OOB_FILL_NONE) == CUDA_SUCCESS;
 }
@@ -1360,7 +1347,7 @@ bool map_mn(CUtensorMap* m, const void* base, long long cols, long long krows, l
   cuuint64_t dims[3] = {64, (cuuint64_t)krows, (cuuint64_t)(cols / 64)};
   cuuint64_t strides[2] = {(cuuint64_t)ld * 2, 128};
   cuuint32_t box[3] = {64, (cuuint32_t)kBK, (cuuint32_t)npanels}, es[3] = {1, 1, 1};
-  return encode_fn3()(m, CU_TENSOR_MAP_DATA_TYPE_FLOAT16, 3, const_cast<void*>(base), dims, strides, box, es,
+  return tensor_map_encode_fn()(m, CU_TENSOR_MAP_DATA_TYPE_FLOAT16, 3, const_cast<void*>(base), dims, strides, box, es,
                       CU_TENSOR_MAP_INTERLEAVE_NONE, CU_TENSOR_MAP_SWIZZLE_128B, CU_TENSOR_MAP_L2_PROMOTION_L2_256B,
                       CU_TENSOR_MAP_FLOAT_OOB_FILL_NONE) == CUDA_SUCCESS;
 }
@@ -1531,7 +1518,7 @@ cudaError_t dib_int16_convert(const float* src, void* dst16, long long n, int bf
 // g_out[M x N] = act(g_in[M x K] W16[K x N] + bias)
 cudaError_t dib_int16_fwd(const void* g_in, int ld_in, const void* w16, const float* bias, void* g_out, int ld_out, int M,
                           int K, int N, int act, float alpha, int bf16, cudaStream_t st) {
-  if (!encode_fn3()) return cudaErrorNotSupported;
+  if (!tensor_map_encode_fn()) return cudaErrorNotSupported;
   CUtensorMap mA, mB;
   if (!map_k(&mA, g_in, K, M, ld_in, kBM) || !map_mn(&mB, w16, N, K, N, kBN / 64))
     return cudaErrorInvalidValue;
@@ -1553,7 +1540,7 @@ cudaError_t dib_int16_fwd(const void* g_in, int ld_in, const void* w16, const fl
 // dz_in[M x K] = (dz[M x N] W16[K x N]^T) * act'(g_in[M x K])      (g_in may be null: no activation, e.g. d_emb)
 cudaError_t dib_int16_dgrad(const void* dz, int ld_dz, const void* w16, const void* g_in, int ld_g, void* dz_in, int ld_out,
                             int M, int K, int N, int act, float alpha, float* colsum_part, int bf16, cudaStream_t st) {
-  if (!encode_fn3()) return cudaErrorNotSupported;
+  if (!tensor_map_encode_fn()) return cudaErrorNotSupported;
   CUtensorMap mA, mB;
   if (!map_k(&mA, dz, N, M, ld_dz, kBM) || !map_k(&mB, w16, N, K, N, kBN))
     return cudaErrorInvalidValue;
@@ -1575,7 +1562,7 @@ cudaError_t dib_int16_dgrad(const void* dz, int ld_dz, const void* w16, const vo
 // dW[K x N] (fp32 split partials, * out_scale) = g_in[M x K]^T dz[M x N];  db = colsum dz
 cudaError_t dib_int16_wgrad(const void* g_in, int ld_g, const void* dz, int ld_dz, float* dW_part, float* db_part, int M, int K,
                             int N, int nsplit, int rows_per_split, long long split_stride, float out_scale, int bf16, cudaStream_t st) {
-  if (!encode_fn3()) return cudaErrorNotSupported;
+  if (!tensor_map_encode_fn()) return cudaErrorNotSupported;
   CUtensorMap mA, mB;
   if (!map_mn(&mA, g_in, K, M, ld_g, kBM / 64) || !map_mn(&mB, dz, N, M, ld_dz, kBN / 64))
     return cudaErrorInvalidValue;
@@ -1607,7 +1594,7 @@ cudaError_t dib_int16_fwd2_head(const void* g_in, int ld_in, int K0, const void*
                                 void* g1, const float* wout, const float* bout, int act, int out_act, float alpha, int loss, const float* y,
                                 int M, float inv_batch, float gscale, void* dg2, float* user_pred, float* wpart, int wpart_stride,
                                 float* loss_part, float* acc_part, int* nblocks, int bf16, cudaStream_t st) {
-  if (!encode_fn3()) return cudaErrorNotSupported;
+  if (!tensor_map_encode_fn()) return cudaErrorNotSupported;
   if (!g_num_sms16) { int dev = 0; cudaGetDevice(&dev); cudaDeviceGetAttribute(&g_num_sms16, cudaDevAttrMultiProcessorCount, dev); }
   CUtensorMap mA, mW0, mW1;
   if (!map_k(&mA, g_in, K0, M, ld_in, kBM) || !map_mn(&mW0, w16_0, kF2N, K0, kF2N, kF2N / 64) || !map_mn(&mW1, w16_1, kF2N, kF2N, kF2N, kF2N / 64))
@@ -1650,7 +1637,7 @@ cudaError_t dib_int16_fwd2_head(const void* g_in, int ld_in, int K0, const void*
 cudaError_t dib_int16_wgrad_pair(const void* g_in0, int K0, const void* dz0, int N0, float* dW_part0, int nsplit0, int rps0,
                                  const void* g_in1, int K1, const void* dz1, int N1, float* dW_part1, int nsplit1, int rps1,
                                  int M, long long split_stride, float out_scale, int bf16, cudaStream_t st) {
-  if (!encode_fn3()) return cudaErrorNotSupported;
+  if (!tensor_map_encode_fn()) return cudaErrorNotSupported;
   CUtensorMap mA, mB, mA2, mB2;
   if (!map_mn(&mA, g_in0, K0, M, K0, kBM / 64) || !map_mn(&mB, dz0, N0, M, N0, kBN / 64) ||
       !map_mn(&mA2, g_in1, K1, M, K1, kBM / 64) || !map_mn(&mB2, dz1, N1, M, N1, kBN / 64))

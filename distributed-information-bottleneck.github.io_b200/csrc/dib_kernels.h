@@ -90,6 +90,11 @@ cudaError_t dib_launch_similarity(int kind, const float* e1, int64_t n, const fl
                                   float* out, cudaStream_t st);
 cudaError_t dib_launch_infonce_head(int kind, const float* e1, const float* e2, int64_t n, int d, float temperature,
                                     float* scratch, float* out_loss, float* d_e1, float* d_e2, cudaStream_t st);
+// streaming tcgen05 head (dib_infonce_tc.cu): kinds 0 l2sq | 1 l2 | 4 cosine, d <= 256, scratch O(n d)
+size_t dib_infonce_head_tc_scratch(int64_t n, int d);
+bool dib_infonce_head_tc_available();
+cudaError_t dib_launch_infonce_head_tc(int kind, const float* e1, const float* e2, int64_t n, int d, float temperature,
+                                       void* scratch, float* out_loss, float* d_e1, float* d_e2, cudaStream_t st);
 
 cudaError_t dib_launch_metrics_update(const float* stats, const float* beta_dev, float* acc, int F, float kl_exponent,
                                       float kl_scale, cudaStream_t st);

@@ -2,10 +2,27 @@
 // kernels: mbarrier, TMA (cp.async.bulk.tensor), tcgen05 (TMEM alloc / mma / commit / ld) and the UMMA shared-memory
 // and instruction descriptors.  Bit layouts follow the PTX ISA / CUTLASS cute/arch/mma_sm100_desc.hpp.
 #pragma once
+#include <cuda.h>
 #include <cuda_runtime.h>
 #include <stdint.h>
 
 namespace sm100 {
+
+// cuTensorMapEncodeTiled through the runtime's driver entry point (no -lcuda link); nullptr where the driver lacks it
+typedef CUresult (*EncodeTiledFn)(CUtensorMap*, CUtensorMapDataType, cuuint32_t, void*, const cuuint64_t*,
+                                  const cuuint64_t*, const cuuint32_t*, const cuuint32_t*, CUtensorMapInterleave,
+                                  CUtensorMapSwizzle, CUtensorMapL2promotion, CUtensorMapFloatOOBfill);
+inline EncodeTiledFn tensor_map_encode_fn() {
+  static EncodeTiledFn fn = nullptr;
+  if (!fn) {
+    void* p = nullptr;
+    cudaDriverEntryPointQueryResult q;
+    if (cudaGetDriverEntryPoint("cuTensorMapEncodeTiled", &p, cudaEnableDefault, &q) == cudaSuccess &&
+        q == cudaDriverEntryPointSuccess)
+      fn = reinterpret_cast<EncodeTiledFn>(p);
+  }
+  return fn;
+}
 
 __device__ __forceinline__ uint32_t smem_u32(const void* p) { return (uint32_t)__cvta_generic_to_shared(p); }
 

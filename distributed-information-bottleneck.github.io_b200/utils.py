@@ -168,23 +168,56 @@ def get_scaled_similarity(embeddings1, embeddings2, similarity_type, temperature
     return out if isinstance(embeddings1, torch.Tensor) else out.cpu().numpy()
 
 
-def infonce_loss_and_grads(embeddings1, embeddings2, similarity_type, temperature, want_grads=True):
-    """The InfoNCE head of the custom loop (train.py:203-213) with its reverse mode (dib_infonce_head).
-    Returns (loss [1], d loss/d embeddings1, d loss/d embeddings2) as device tensors (grads None if not wanted)."""
-    kind = _similarity_kind(similarity_type)
-    lib = _lib.load()
+# the exact head (dib_infonce_head) keeps the n x n similarity matrix in scratch and stops here
+_EXACT_HEAD_MAX_N = 32768
+# similarities with a Gram form, which the streaming tensor-core head (dib_infonce_head_tc) computes
+_GRAM_KINDS = (SIMILARITY_TYPES["l2sq"], SIMILARITY_TYPES["l2"], SIMILARITY_TYPES["cosine"])
+
+
+def _infonce_inputs(embeddings1, embeddings2):
     device = (embeddings1.device if isinstance(embeddings1, torch.Tensor) and embeddings1.is_cuda
               else torch.device("cuda", torch.cuda.current_device()))
     e1, e2 = _dev(embeddings1, device), _dev(embeddings2, device)
     if e1.shape != e2.shape:
         raise ValueError("the InfoNCE loss needs two [n, d] batches of equal shape (train.py:222-223)")
-    n, d = e1.shape
-    scratch = torch.empty(n * n + 4 * n, dtype=torch.float32, device=device)
     loss = torch.empty(1, dtype=torch.float32, device=device)
+    return device, e1, e2, loss
+
+
+def infonce_loss_and_grads(embeddings1, embeddings2, similarity_type, temperature, want_grads=True):
+    """The InfoNCE head of the custom loop (train.py:203-213) with its reverse mode (dib_infonce_head).
+    Returns (loss [1], d loss/d embeddings1, d loss/d embeddings2) as device tensors (grads None if not wanted).
+    Batches above 32768 rows, where the exact head's n x n scratch no longer fits, run on the streaming tensor-core head
+    (dib_infonce_head_tc) for 'l2sq', 'l2' and 'cosine'; 'l1' and 'linf' have no such path and raise there."""
+    kind = _similarity_kind(similarity_type)
+    lib = _lib.load()
+    device, e1, e2, loss = _infonce_inputs(embeddings1, embeddings2)
+    n, d = e1.shape
+    if n > _EXACT_HEAD_MAX_N and kind in _GRAM_KINDS:
+        return _infonce_head_tc(e1, e2, kind, temperature, want_grads)
+    scratch = torch.empty(n * n + 4 * n, dtype=torch.float32, device=device)
     d1 = torch.empty_like(e1) if want_grads else None
     d2 = torch.empty_like(e2) if want_grads else None
     with torch.cuda.device(device):
         _lib.check(lib.dib_infonce_head(kind, _lib.ptr(e1), _lib.ptr(e2), n, d, float(temperature), _lib.ptr(scratch),
                                         _lib.ptr(loss), _lib.ptr(d1), _lib.ptr(d2),
                                         ctypes.c_void_p(torch.cuda.current_stream().cuda_stream)))
+    return loss, d1, d2
+
+
+def _infonce_head_tc(embeddings1, embeddings2, kind, temperature, want_grads=True):
+    """dib_infonce_head_tc at any n: the same (loss, d_e1, d_e2) as dib_infonce_head, streamed on the tensor cores."""
+    lib = _lib.load()
+    device, e1, e2, loss = _infonce_inputs(embeddings1, embeddings2)
+    n, d = e1.shape
+    nbytes = lib.dib_infonce_head_tc_scratch_bytes(n, d)
+    if nbytes < 0:
+        raise ValueError(f"the tensor-core InfoNCE head takes 1 <= n <= 2^26 rows of d <= 256 (got n={n}, d={d})")
+    scratch = torch.empty(nbytes, dtype=torch.uint8, device=device)
+    d1 = torch.empty_like(e1) if want_grads else None
+    d2 = torch.empty_like(e2) if want_grads else None
+    with torch.cuda.device(device):
+        _lib.check(lib.dib_infonce_head_tc(kind, _lib.ptr(e1), _lib.ptr(e2), n, d, float(temperature), _lib.ptr(scratch),
+                                           _lib.ptr(loss), _lib.ptr(d1), _lib.ptr(d2),
+                                           ctypes.c_void_p(torch.cuda.current_stream().cuda_stream)))
     return loss, d1, d2

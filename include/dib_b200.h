@@ -247,6 +247,15 @@ int dib_scaled_similarity(int32_t kind, const float* e1, int64_t n, const float*
 int dib_infonce_head(int32_t kind, const float* e1, const float* e2, int64_t n, int32_t d, float temperature,
                      float* scratch, float* out_loss, float* d_e1, float* d_e2, void* stream);
 
+/* The same head, streamed on the tensor cores (tcgen05) for the similarities with a Gram form: kind 0 'l2sq' | 1 'l2' |
+ * 4 'cosine'.  The n x n similarity matrix is never stored: scratch is O(n d) bytes, as returned by
+ * dib_infonce_head_tc_scratch_bytes (-1 for arguments out of range), and must be 128-byte aligned.  1 <= n <= 2^26,
+ * 1 <= d <= 256.  Products use bf16 hi + lo split operands with fp32 accumulation, the positive pairs s_ii are exact
+ * fp32; deterministic (identical calls give identical bytes).  No allocation, no host synchronisation. */
+int64_t dib_infonce_head_tc_scratch_bytes(int64_t n, int32_t d);
+int dib_infonce_head_tc(int32_t kind, const float* e1, const float* e2, int64_t n, int32_t d, float temperature,
+                        void* scratch, float* out_loss, float* d_e1, float* d_e2, void* stream);
+
 /* NEXT ROW f1 -- utils.estimate_mi_sandwich_bounds' per-batch kernel (utils.py:36-65): InfoNCE lower and leave-one-out
  * upper bound (nats) of I(U;X) for one encoder on one batch of n samples.  mu_logvar [n, 2E] (dib_encode_feature
  * output); eps [n, E] or NULL -> Philox(seed, step, row, feature 0, dim); row_scratch [2n] floats; out [2]. */
