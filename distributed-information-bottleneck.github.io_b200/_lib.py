@@ -9,7 +9,9 @@ from . import build as _build
 ABI_VERSION = 2
 
 ACTIVATIONS = {None: 0, "linear": 0, "relu": 1, "tanh": 2, "leaky_relu": 3, "sigmoid": 4, "elu": 5}
-LOSSES = {"bce_logits": 0, "sparse_ce_logits": 1, "mse": 2, "external": 3, "bce_probs": 4}
+LOSSES = {"bce_logits": 0, "sparse_ce_logits": 1, "mse": 2, "external": 3, "bce_probs": 4, "infonce": 5}
+# similarity_type of utils.get_scaled_similarity (utils.py:127-175) -> the `kind` of the InfoNCE entry points
+SIMILARITIES = {"l2sq": 0, "l2": 1, "l1": 2, "linf": 3, "cosine": 4}
 ENCODER_KINDS = {"mlp": 0, "simple": 1}
 # 'fp16' / 'bf16': fused 16-bit-operand tcgen05 kernels (fp32 accumulate); 'tf32': kind::tf32 GEMMs on fp32 storage;
 # 'fp32': exact CUDA-core FMA parity path.  See enum dib_precision in include/dib_b200.h.
@@ -40,6 +42,14 @@ class DibConfig(ctypes.Structure):
         ("kl_loss_scale", c_float),
         ("encoder_kind", c_int32),
         ("dropout_rate", c_float),
+    ]
+
+
+class DibOutputEncoderConfig(ctypes.Structure):
+    _fields_ = [
+        ("input_dimensionality", c_int32),
+        ("number_layers", c_int32),
+        ("architecture", POINTER(c_int32)),
     ]
 
 
@@ -80,6 +90,15 @@ SIGNATURES = {
     "dib_infonce_head_tc_scratch_bytes": (c_int64, [c_int64, c_int32]),
     "dib_infonce_head_tc": (c_int32, [c_int32, c_void_p, c_void_p, c_int64, c_int32, c_float, c_void_p, c_void_p, c_void_p,
                                       c_void_p, c_void_p]),
+    "dib_attach_output_encoder": (c_int32, [c_void_p, POINTER(DibOutputEncoderConfig)]),
+    "dib_output_encoder_param_count": (c_int64, [c_void_p]),
+    "dib_output_encoder_param_layout": (c_int32, [c_void_p, POINTER(c_int64), POINTER(c_int32), POINTER(c_int32), c_int32]),
+    "dib_output_encoder_forward": (c_int32, [c_void_p, c_void_p, c_void_p, c_int64, c_void_p, c_void_p, c_void_p]),
+    "dib_infonce_train_step": (c_int32, [c_void_p, c_void_p, c_void_p, c_void_p, c_int64, c_void_p, c_int32, c_float, c_void_p,
+                                         c_uint64, c_uint32, c_uint64, c_void_p, c_void_p, c_void_p, c_void_p, c_void_p]),
+    "dib_infonce_forward": (c_int32, [c_void_p, c_void_p, c_void_p, c_void_p, c_int64, c_void_p, c_int32, c_float, c_void_p,
+                                      c_uint64, c_uint32, c_uint64, c_void_p, c_void_p, c_void_p, c_void_p]),
+    "dib_infonce_scratch_bytes": (c_int64, [c_int32, c_int64, c_int32]),
     "dib_ctw_estimate_entropy": (c_int32, [c_void_p, c_int64, c_int32, c_void_p]),
     "dib_ctw_estimate_entropy_batch": (c_int32, [c_void_p, c_void_p, c_int32, c_int32, c_int32, c_void_p]),
     "dib_ctw_last_error": (c_char_p, []),

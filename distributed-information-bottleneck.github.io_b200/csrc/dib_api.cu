@@ -90,6 +90,23 @@ struct dib_model {
   bool simple = false;                 // nb-bool SimpleEncoder: two (1,1) constants per feature
   int* d_xoff = nullptr;               // device copy of x_off (simple-encoder kernels)
   long long beta_eff_off = 0;          // one float in the workspace: d(beta*scale*KL^p)/dKL
+  // output encoder of a DIB_LOSS_INFONCE handle (train.py:186-193; dib_attach_output_encoder).  Its Q parameters sit at
+  // params[P, P+Q) in Keras order; the GEMMs read them from a shadow in the workspace with every variable 4-float aligned:
+  // [W0 | W1 | ... | b0 | b1 | ...] (the kernels TF32-rounded in the tensor-core modes)
+  bool oe = false;
+  int oe_dy = 0, oe_L = 0, oe_ldpe = 0;
+  std::vector<int> oe_arch;
+  long long Q = 0, oe_wlen = 0, oe_shadow_len = 0, oe_part_stride = 0;
+  std::vector<long long> oe_var_off;                // relative to P, Keras order
+  std::vector<int> oe_var_rows, oe_var_cols;
+  std::vector<long long> oeW, oeB;                  // per layer: shadow / partial-row offsets
+  Buf oe_pe, oe_out, oe_dout;
+  std::vector<Buf> oe_act, oe_d;                    // index 1..oe_L
+  long long oe_shadow_off = 0, oe_part_off = 0, oe_cont_off = 0, nce_loss_off = 0;
+  int* d_oe_col_src = nullptr;
+  int* d_oe_col_freq = nullptr;
+  std::vector<int> oe_fwd, oe_dgrad, oe_wgrad;
+  DibOePackTable oe_pack;
   // optional per-launch-group timing with CUDA events on the caller's stream (dib_profile_*)
   bool profiling = false;
   struct ProfRec { std::string label; cudaEvent_t a, b; };
@@ -107,6 +124,8 @@ int enc_fan_in(const dib_model* h, int f, int j) { return j == 0 ? h->w_in[f] : 
 int enc_fan_out(const dib_model* h, int j) { return j < h->L ? h->enc_arch[j] : 2 * h->E; }
 int int_fan_in(const dib_model* h, int j) { return j == 0 ? h->F * h->E : h->int_arch[j - 1]; }
 int int_fan_out(const dib_model* h, int j) { return j < h->Li ? h->int_arch[j] : h->out; }
+int oe_fan_in(const dib_model* h, int j) { return j == 0 ? h->oe_dy * h->nfreq : h->oe_arch[j - 1]; }
+int oe_fan_out(const dib_model* h, int j) { return j < h->oe_L ? h->oe_arch[j] : h->out; }
 
 long long take(long long& cursor, long long floats) {
   const long long off = cursor;
@@ -177,6 +196,19 @@ void plan(dib_model* h) {
   h->beta_eff_off = take(c, 64);
   h->wshadow_off = take(c, h->Pp);      // TF32-rounded copy of the parameters (tensor-core mode B operands)
   h->pack_off = take(c, (long long)(dib_enc_fused_pack_bytes(h->F) + 3) / 4);
+  if (h->oe) {
+    h->oe_pe = make_buf(c, B, h->oe_ldpe, 1);
+    h->oe_act.assign(h->oe_L + 1, Buf());
+    h->oe_d.assign(h->oe_L + 1, Buf());
+    for (int j = 1; j <= h->oe_L; ++j) h->oe_act[j] = make_buf(c, B, h->oe_arch[j - 1], 1);
+    h->oe_out = make_buf(c, B, h->out, 1);
+    h->oe_dout = make_buf(c, B, h->out, 1);
+    for (int j = 1; j <= h->oe_L; ++j) h->oe_d[j] = make_buf(c, B, h->oe_arch[j - 1], 1);
+    h->oe_shadow_off = take(c, h->oe_shadow_len);
+    h->oe_part_off = take(c, (long long)kMaxSplits * h->oe_part_stride);
+    h->oe_cont_off = take(c, 4 * B * h->out);    // unpadded [n, D] e1 | e2 | d e1 | d e2 for the heads
+    h->nce_loss_off = take(c, 64);
+  }
   h->ws_floats = c;
 }
 
@@ -275,6 +307,49 @@ void build_problems(dib_model* h, std::vector<DibGemmProblem>& v) {
     p.R = int_fan_in(h, j); p.C = int_fan_out(h, j);
     v.push_back(p);
   }
+  if (!h->oe) return;
+  // output encoder: weights / biases / weight gradients are offsets into its shadow and its partial rows (gemm_oe)
+  const int Lo = h->oe_L;
+  h->oe_fwd.assign(Lo + 1, -1); h->oe_dgrad.assign(Lo + 1, -1); h->oe_wgrad.assign(Lo + 1, -1);
+  auto oeA = [&](int j, long long& off, int& ld) {
+    const Buf& b = j == 0 ? h->oe_pe : h->oe_act[j];
+    off = b.off; ld = b.ld;
+  };
+  auto oeDZ = [&](int j, long long& off, int& ld) {
+    const Buf& b = j == Lo ? h->oe_dout : h->oe_d[j + 1];
+    off = b.off; ld = b.ld;
+  };
+  for (int j = 0; j <= Lo; ++j) {
+    h->oe_fwd[j] = (int)v.size();
+    DibGemmProblem p = zero();
+    oeA(j, p.a_off, p.lda);
+    p.b_off = h->oeW[j]; p.ldb = oe_fan_out(h, j);
+    const Buf& o = j < Lo ? h->oe_act[j + 1] : h->oe_out;
+    p.c_off = o.off; p.ldc = o.ld;
+    p.x_off = h->oeB[j];
+    p.T = oe_fan_in(h, j); p.C = oe_fan_out(h, j); p.act = j < Lo ? h->act : DIB_ACT_LINEAR;
+    v.push_back(p);
+  }
+  for (int j = 1; j <= Lo; ++j) {
+    h->oe_dgrad[j] = (int)v.size();
+    DibGemmProblem p = zero();
+    oeDZ(j, p.a_off, p.lda);
+    p.b_off = h->oeW[j]; p.ldb = oe_fan_out(h, j);
+    p.c_off = h->oe_d[j].off; p.ldc = h->oe_d[j].ld;
+    p.x_off = h->oe_act[j].off; p.ldx = h->oe_act[j].ld; p.act = h->act;
+    p.T = oe_fan_out(h, j); p.C = oe_fan_in(h, j);
+    v.push_back(p);
+  }
+  for (int j = 0; j <= Lo; ++j) {
+    h->oe_wgrad[j] = (int)v.size();
+    DibGemmProblem p = zero();
+    oeA(j, p.a_off, p.lda);
+    oeDZ(j, p.b_off, p.ldb);
+    p.c_off = h->oeW[j]; p.ldc = oe_fan_out(h, j);
+    p.x_off = h->oeB[j];
+    p.R = oe_fan_in(h, j); p.C = oe_fan_out(h, j);
+    v.push_back(p);
+  }
 }
 
 struct Ctx {
@@ -326,6 +401,72 @@ int gemm(const Ctx& c, int mode, int first, int nprob, int maxC, int maxR, int n
   return 0;
 }
 
+// one output-encoder layer: the same kernels as gemm(), with the weights and biases read from the encoder's aligned shadow
+// and the weight-gradient partials written to its own partial rows
+int gemm_oe(const Ctx& c, int mode, int first, int maxC, int maxR, int nsplit, int rps) {
+  dib_model* h = c.h;
+  DibGemmLaunch L;
+  L.probs = h->d_probs + first;
+  L.nprob = 1;
+  L.M = c.n;
+  L.maxC = maxC; L.maxR = maxR;
+  L.nsplit = nsplit; L.rows_per_split = rps; L.split_stride = h->oe_part_stride;
+  L.alpha = h->alpha;
+  const bool tc = is_tc(h);
+  L.round_out = tc ? 1 : 0;
+  float* sh = c.ws + h->oe_shadow_off;
+  float* part = c.ws + h->oe_part_off;
+  switch (mode) {
+    case DIB_GEMM_FWD: L.baseA = c.ws; L.baseB = sh; L.baseC = c.ws; L.baseX = nullptr; L.baseBias = sh; break;
+    case DIB_GEMM_DGRAD: L.baseA = c.ws; L.baseB = sh; L.baseC = c.ws; L.baseX = c.ws; break;
+    default: L.baseA = c.ws; L.baseB = c.ws; L.baseC = part; L.baseX = part; break;
+  }
+  if (tc && dib_gemm_tc_eligible(mode, h->h_probs.data() + first, 1, sh)) {
+    DIB_CUDA_OK(dib_launch_gemm_tc(mode, L, h->h_probs.data() + first, c.st));
+    return 0;
+  }
+  DIB_CUDA_OK(dib_launch_gemm_simt(mode, L, c.st));
+  return 0;
+}
+
+// output_encoder(y) (train.py:186-193) on n rows into the oe_out workspace buffer
+int oe_forward(const Ctx& c, const float* y) {
+  dib_model* h = c.h;
+  const int rnd = is_tc(h) ? 1 : 0;
+  prof_begin(c, "oe_fwd");
+  DIB_CUDA_OK(dib_launch_oe_pack(c.params + h->P, c.ws + h->oe_shadow_off, h->oe_pack, c.st));
+  DIB_CUDA_OK(dib_launch_pe(y, h->oe_dy, 0, h->d_oe_col_src, h->d_oe_col_freq, 0, h->oe_ldpe, c.ws + h->oe_pe.off, h->oe_ldpe, 0,
+                            c.n, rnd, c.st));
+  for (int j = 0; j <= h->oe_L; ++j)
+    if (gemm_oe(c, DIB_GEMM_FWD, h->oe_fwd[j], oe_fan_out(h, j), 0, 1, 0)) return 1;
+  prof_end(c);
+  return 0;
+}
+
+// reverse mode of oe_forward from d e2 in oe_dout (the shadow and the activations as oe_forward left them) ->
+// grads_q [Q] in Keras order
+int oe_backward(const Ctx& c, int nsplit, int rps, float* grads_q) {
+  dib_model* h = c.h;
+  prof_begin(c, "oe_bwd");
+  for (int j = h->oe_L; j >= 0; --j) {
+    if (gemm_oe(c, DIB_GEMM_WGRAD, h->oe_wgrad[j], oe_fan_out(h, j), oe_fan_in(h, j), nsplit, rps)) return 1;
+    if (j >= 1 && gemm_oe(c, DIB_GEMM_DGRAD, h->oe_dgrad[j], oe_fan_in(h, j), 0, 1, 0)) return 1;
+  }
+  // fixed-order sums of the batch-split partials, written straight to the Keras-ordered gradient
+  const float* part = c.ws + h->oe_part_off;
+  std::vector<DibReduceSeg> segs;
+  for (int v = 0; v < h->oe_pack.nvar; ++v) {
+    segs.push_back({part + h->oe_pack.dst_off[v], h->oe_part_stride, nsplit, h->oe_pack.count[v], 1.f,
+                    grads_q + h->oe_pack.src_off[v]});
+    if ((int)segs.size() == kDibMaxReduceSegs || v + 1 == h->oe_pack.nvar) {
+      DIB_CUDA_OK(dib_launch_reduce_segments(segs.data(), (int)segs.size(), c.st));
+      segs.clear();
+    }
+  }
+  prof_end(c);
+  return 0;
+}
+
 int check_call(const dib_model* h, const void* params, const void* x, int64_t n, const void* ws) {
   if (!h) return fail("null model handle");
   if (!params || !ws || (!x && n > 0)) return fail("null params / x / workspace pointer");
@@ -339,9 +480,28 @@ int check_call(const dib_model* h, const void* params, const void* x, int64_t n,
 struct NoiseKey { uint64_t seed; uint32_t step; uint64_t sample_offset; bool training; };
 int encode_all(const Ctx& c, const float* x, int ldx, int rnd, const int* row_index, int64_t n_src, const NoiseKey* key = nullptr);
 
+// the compiled loss on the prediction in the pred buffer (d_pred when training) and the statistics vector.  A
+// DIB_LOSS_INFONCE handle runs the external-loss branch: y is then d L_infonce / d e1.
+int loss_and_stats(const Ctx& c, const float* y, float inv_batch, bool training, float* user_pred, float* out_stats, int nblk_kl) {
+  dib_model* h = c.h;
+  const int rnd = is_tc(h) ? 1 : 0;
+  const int loss = h->loss == DIB_LOSS_INFONCE ? DIB_LOSS_EXTERNAL : h->loss;
+  prof_begin(c, "loss_stats");
+  DIB_CUDA_OK(dib_launch_loss(loss, h->out_act, h->alpha, c.ws + h->pred.off, h->pred.ld, y, h->out, c.n, inv_batch,
+                              training ? c.ws + h->d_pred.off : nullptr, user_pred, c.ws + h->loss_part_off,
+                              c.ws + h->acc_part_off, rnd, c.st));
+  const int nblk = (int)DIB_CEIL_DIV((long long)c.n, (long long)kRowsPerBlock);
+  DIB_CUDA_OK(dib_launch_finalize_stats(c.ws + h->kl_part_off, h->kl_stride, nblk_kl, c.ws + h->loss_part_off,
+                                        c.ws + h->acc_part_off, nblk, h->F, c.n, y != nullptr, out_stats, c.st));
+  prof_end(c);
+  return 0;
+}
+
+// stop_nblk_kl != nullptr: stop after the integration network (the prediction is in the pred buffer) and return the KL
+// partial count that loss_and_stats needs -- the InfoNCE step computes the loss gradient in between
 int run_forward(const Ctx& c, const float* x, const float* y, const float* eps, uint64_t seed, uint32_t step,
                 uint64_t sample_offset, float inv_batch, bool training, float* user_pred, float* user_emb,
-                float* out_stats, bool enc_only = false) {
+                float* out_stats, bool enc_only = false, int* stop_nblk_kl = nullptr) {
   dib_model* h = c.h;
   const int rnd = is_tc(h) ? 1 : 0;
   const bool fast_path = h->fused_ok && rnd && (!training || h->fused_bwd_ok) && !h->force_unfused && h->int16_ok && !h->force_int32;
@@ -460,15 +620,8 @@ int run_forward(const Ctx& c, const float* x, const float* y, const float* eps, 
     if (gemm(c, DIB_GEMM_FWD, h->int_fwd[j], 1, int_fan_out(h, j), 0, 1, 0)) return 1;
     prof_end(c);
   }
-  prof_begin(c, "loss_stats");
-  DIB_CUDA_OK(dib_launch_loss(h->loss, h->out_act, h->alpha, c.ws + h->pred.off, h->pred.ld, y, h->out, c.n, inv_batch,
-                              training ? c.ws + h->d_pred.off : nullptr, user_pred, c.ws + h->loss_part_off,
-                              c.ws + h->acc_part_off, rnd, c.st));
-  const int nblk = (int)DIB_CEIL_DIV((long long)c.n, (long long)kRowsPerBlock);
-  DIB_CUDA_OK(dib_launch_finalize_stats(c.ws + h->kl_part_off, h->kl_stride, nblk_kl, c.ws + h->loss_part_off,
-                                        c.ws + h->acc_part_off, nblk, h->F, c.n, y != nullptr, out_stats, c.st));
-  prof_end(c);
-  return 0;
+  if (stop_nblk_kl) { *stop_nblk_kl = nblk_kl; return 0; }
+  return loss_and_stats(c, y, inv_batch, training, user_pred, out_stats, nblk_kl);
 }
 
 // every feature encoder on n rows of x (deterministic part: mu | logvar incl. the offset) into the enc_out workspace
@@ -616,6 +769,13 @@ int32_t dib_model_info(const dib_model* h, char* out, size_t out_bytes) {
     s += fused ? std::string(" operands=") + (h->precision == DIB_PREC_BF16 ? "bf16" : "fp16") : std::string(" operands=tf32");
     s += " accumulate=fp32";
   }
+  if (h->oe) {      // the kernel family of each output-encoder layer (narrow first layers stay on the SIMT kernel)
+    s += " output_encoder=";
+    for (int j = 0; j <= h->oe_L; ++j) {
+      const bool tc = is_tc(h) && dib_gemm_tc_eligible(DIB_GEMM_FWD, &h->h_probs[h->oe_fwd[j]], 1, nullptr);
+      s += std::string(j ? "," : "") + (tc ? "tcgen05-tf32" : "simt-fp32");
+    }
+  }
   const size_t k = s.size() < out_bytes - 1 ? s.size() : out_bytes - 1;
   memcpy(out, s.data(), k); out[k] = 0;
   return (int32_t)k;
@@ -634,7 +794,9 @@ int dib_create(const dib_config* cfg, dib_model** out) {
   if (cfg->activation_fn < 0 || cfg->activation_fn > DIB_ACT_ELU || cfg->output_activation_fn < 0 ||
       cfg->output_activation_fn > DIB_ACT_ELU)
     return fail("dib_create: unknown activation");
-  if (cfg->loss < 0 || cfg->loss > DIB_LOSS_BCE_PROBS) return fail("dib_create: unknown loss");
+  if (cfg->loss < 0 || cfg->loss > DIB_LOSS_INFONCE) return fail("dib_create: unknown loss");
+  if (cfg->loss == DIB_LOSS_INFONCE && cfg->output_activation_fn != DIB_ACT_LINEAR)
+    return fail("dib_create: DIB_LOSS_INFONCE needs a linear output activation (the model output is the embedding e1)");
   dib_model* h = new (std::nothrow) dib_model();
   if (!h) return fail("dib_create: out of host memory");
   h->F = cfg->number_features; h->L = cfg->number_encoder_layers; h->Li = cfg->number_integration_layers;
@@ -755,7 +917,7 @@ int dib_create(const dib_config* cfg, dib_model** out) {
         // 16-bit integration path: hidden widths multiples of 128, last hidden width 256, narrow output head
         // (the fused head owns the compiled loss, so a caller-owned loss takes the TF32 integration kernels)
         bool iok = h->Li >= 1 && (h->F * h->E) % 64 == 0 && h->int_arch[h->Li - 1] == 256 && h->out <= 16 &&
-                   h->loss != DIB_LOSS_EXTERNAL;
+                   h->loss != DIB_LOSS_EXTERNAL && h->loss != DIB_LOSS_INFONCE;
         for (int j = 0; iok && j < h->Li; ++j) iok = h->int_arch[j] % 128 == 0 && (h->intB[j] & 3) == 0;
         h->int16_ok = iok;
       }
@@ -773,6 +935,8 @@ void dib_destroy(dib_model* h) {
   if (h->d_col_feat) cudaFree(h->d_col_feat);
   if (h->d_xoff) cudaFree(h->d_xoff);
   if (h->d_fused_tables) cudaFree(h->d_fused_tables);
+  if (h->d_oe_col_src) cudaFree(h->d_oe_col_src);
+  if (h->d_oe_col_freq) cudaFree(h->d_oe_col_freq);
   for (auto& r : h->prof) { cudaEventDestroy(r.a); cudaEventDestroy(r.b); }
   delete h;
 }
@@ -798,6 +962,7 @@ int dib_forward(dib_model* h, const float* params, const float* x, const float* 
   (void)beta_dev;
   if (check_call(h, params, x, n, workspace)) return 1;
   if (!out_stats) return fail("dib_forward: out_stats is required");
+  if (h->loss == DIB_LOSS_INFONCE && y) return fail("dib_forward: a DIB_LOSS_INFONCE handle takes y = NULL (the loss needs e2: dib_infonce_forward)");
   Ctx c{h, params, static_cast<float*>(workspace), static_cast<cudaStream_t>(stream), (int)n};
   if (n == 0) { DIB_CUDA_OK(cudaMemsetAsync(out_stats, 0, sizeof(float) * (h->F + 3), c.st)); return 0; }
   return run_forward(c, x, y, eps, seed, step, sample_offset, 0.f, false, out_pred, out_emb, out_stats);
@@ -836,28 +1001,22 @@ int dib_encode_feature(dib_model* h, const float* params, int32_t feature, const
 // phases: 1 = forward + compiled loss + integration-network backward (grads_flat[first integration parameter ..) final),
 //         2 = encoder backward (grads_flat[0 .. first integration parameter) final); 3 = both (= dib_train_step).
 // Phase 2 relies on the workspace exactly as phase 1 left it (same x, eps / seed / step, n).
-int dib_train_step_phased(dib_model* h, const float* params, const float* x, const float* y, int64_t n, const float* beta_dev,
-                          float inv_global_batch, const float* eps, uint64_t seed, uint32_t step, uint64_t sample_offset,
-                          float* grads_flat, float* out_stats, void* workspace, int32_t phases, void* stream) {
-  if (check_call(h, params, x, n, workspace)) return 1;
-  if ((!y && n > 0) || !beta_dev || !grads_flat || !out_stats)
-    return fail("dib_train_step: y, beta_dev, grads_flat and out_stats are required");
-  if (phases < 1 || phases > 3) return fail("dib_train_step_phased: phases must be 1, 2 or 3");
+}  // extern "C"
+
+namespace {
+
+// the body of dib_train_step_phased for n > 0.  forward_done: the caller already ran the forward, the loss gradient into
+// d_pred and out_stats (the InfoNCE step); phase 1 then starts at the IB weight.
+int train_phases(const Ctx& c, const float* x, const float* y, int64_t n, const float* beta_dev, float inv_global_batch,
+                 const float* eps, uint64_t seed, uint32_t step, uint64_t sample_offset, float* grads_flat, float* out_stats,
+                 int32_t phases, bool forward_done) {
+  dib_model* h = c.h;
   const bool phA = (phases & 1) != 0, phB = (phases & 2) != 0;
-  Ctx c{h, params, static_cast<float*>(workspace), static_cast<cudaStream_t>(stream), (int)n};
-  c.dev_step = true;
   const long long p_enc = h->intW[0];                // encoder parameters occupy [0, p_enc)
-  if (n == 0) {
-    if (phB) DIB_CUDA_OK(cudaMemsetAsync(grads_flat, 0, sizeof(float) * p_enc, c.st));
-    if (phA) {
-      DIB_CUDA_OK(cudaMemsetAsync(grads_flat + p_enc, 0, sizeof(float) * (h->P - p_enc), c.st));
-      DIB_CUDA_OK(cudaMemsetAsync(out_stats, 0, sizeof(float) * (h->F + 3), c.st));
-    }
-    return 0;
-  }
   const bool nonlinear = h->kl_exp != 1.f || h->kl_scale != 1.f;
   if (phA) {
-    if (run_forward(c, x, y, eps, seed, step, sample_offset, inv_global_batch, true, nullptr, nullptr, out_stats)) return 1;
+    if (!forward_done &&
+        run_forward(c, x, y, eps, seed, step, sample_offset, inv_global_batch, true, nullptr, nullptr, out_stats)) return 1;
     const float* bw = nullptr;
     if (ib_weight(c, beta_dev, out_stats, inv_global_batch, &bw)) return 1;
   }
@@ -1008,6 +1167,35 @@ int dib_train_step_phased(dib_model* h, const float* params, const float* x, con
   DIB_CUDA_OK(dib_launch_reduce_partials(part, h->Pp, nsplit, p_enc, grads_flat, c.st));
   prof_end(c);
   return 0;
+}
+
+}  // namespace
+
+extern "C" {
+
+int dib_train_step_phased(dib_model* h, const float* params, const float* x, const float* y, int64_t n, const float* beta_dev,
+                          float inv_global_batch, const float* eps, uint64_t seed, uint32_t step, uint64_t sample_offset,
+                          float* grads_flat, float* out_stats, void* workspace, int32_t phases, void* stream) {
+  if (check_call(h, params, x, n, workspace)) return 1;
+  if (h->loss == DIB_LOSS_INFONCE)
+    return fail("dib_train_step: a DIB_LOSS_INFONCE handle trains with dib_infonce_train_step (the step needs the output encoder)");
+  if ((!y && n > 0) || !beta_dev || !grads_flat || !out_stats)
+    return fail("dib_train_step: y, beta_dev, grads_flat and out_stats are required");
+  if (phases < 1 || phases > 3) return fail("dib_train_step_phased: phases must be 1, 2 or 3");
+  const bool phA = (phases & 1) != 0, phB = (phases & 2) != 0;
+  Ctx c{h, params, static_cast<float*>(workspace), static_cast<cudaStream_t>(stream), (int)n};
+  c.dev_step = true;
+  const long long p_enc = h->intW[0];                // encoder parameters occupy [0, p_enc)
+  if (n == 0) {
+    if (phB) DIB_CUDA_OK(cudaMemsetAsync(grads_flat, 0, sizeof(float) * p_enc, c.st));
+    if (phA) {
+      DIB_CUDA_OK(cudaMemsetAsync(grads_flat + p_enc, 0, sizeof(float) * (h->P - p_enc), c.st));
+      DIB_CUDA_OK(cudaMemsetAsync(out_stats, 0, sizeof(float) * (h->F + 3), c.st));
+    }
+    return 0;
+  }
+  return train_phases(c, x, y, n, beta_dev, inv_global_batch, eps, seed, step, sample_offset, grads_flat, out_stats, phases,
+                      false);
 }
 
 int dib_train_step(dib_model* h, const float* params, const float* x, const float* y, int64_t n, const float* beta_dev,
@@ -1250,6 +1438,189 @@ int dib_compression_matrices(dib_model* h, const float* params, const float* x, 
     DIB_CUDA_OK(dib_launch_pairwise_gauss(0, eo, h->enc_out.ld, h->enc_out.feat_stride, n, eo, h->enc_out.ld,
                                           h->enc_out.feat_stride, n, h->E, h->F, out_dist, out_compression, c.st));
   return 0;
+}
+
+// ---- InfoNCE training (train.py:180-289) ------------------------------------------------------------------------------
+int dib_attach_output_encoder(dib_model* h, const dib_output_encoder_config* cfg) {
+  if (!h || !cfg) return fail("dib_attach_output_encoder: null argument");
+  if (h->loss != DIB_LOSS_INFONCE) return fail("dib_attach_output_encoder: the handle was not created with DIB_LOSS_INFONCE");
+  if (h->oe) return fail("dib_attach_output_encoder: an output encoder is already attached");
+  if (cfg->input_dimensionality < 1 || cfg->number_layers < 0 || cfg->number_layers > kDibMaxOeLayers ||
+      (cfg->number_layers > 0 && !cfg->architecture))
+    return fail("dib_attach_output_encoder: bad sizes (input_dimensionality >= 1, 0 <= number_layers <= " +
+                std::to_string(kDibMaxOeLayers) + ")");
+  for (int j = 0; j < cfg->number_layers; ++j)
+    if (cfg->architecture[j] < 1) return fail("dib_attach_output_encoder: width < 1");
+  h->oe_dy = cfg->input_dimensionality;
+  h->oe_L = cfg->number_layers;
+  h->oe_arch.assign(cfg->architecture, cfg->architecture + h->oe_L);
+  // PE of y with the model's frequencies (train.py:187-189), columns padded to a multiple of 4
+  std::vector<int> col_src, col_freq;
+  for (int blk = 0; blk < h->nfreq; ++blk)
+    for (int k = 0; k < h->oe_dy; ++k) { col_src.push_back(k); col_freq.push_back(blk == 0 ? 0 : (1 << blk)); }
+  while (col_src.size() % 4) { col_src.push_back(-1); col_freq.push_back(0); }
+  h->oe_ldpe = (int)col_src.size();
+  // Keras-ordered parameters and their aligned shadow: kernels first (one TF32 rounding range), then biases
+  h->oe_var_off.clear(); h->oe_var_rows.clear(); h->oe_var_cols.clear();
+  h->oeW.assign(h->oe_L + 1, 0); h->oeB.assign(h->oe_L + 1, 0);
+  long long off = 0, sh = 0;
+  for (int j = 0; j <= h->oe_L; ++j) {
+    const long long fi = oe_fan_in(h, j), fo = oe_fan_out(h, j);
+    h->oe_var_off.push_back(off); h->oe_var_rows.push_back((int)fi); h->oe_var_cols.push_back((int)fo); off += fi * fo;
+    h->oe_var_off.push_back(off); h->oe_var_rows.push_back(0); h->oe_var_cols.push_back((int)fo); off += fo;
+    h->oeW[j] = sh; sh += DIB_ROUND_UP(fi * fo, 4ll);
+  }
+  h->oe_wlen = sh;
+  for (int j = 0; j <= h->oe_L; ++j) { h->oeB[j] = sh; sh += DIB_ROUND_UP((long long)oe_fan_out(h, j), 4ll); }
+  h->Q = off; h->oe_shadow_len = sh; h->oe_part_stride = DIB_ROUND_UP(sh, 64ll);
+  DibOePackTable& t = h->oe_pack;
+  t.nvar = 2 * (h->oe_L + 1);
+  for (int j = 0; j <= h->oe_L; ++j) {
+    t.src_off[2 * j] = h->oe_var_off[2 * j]; t.dst_off[2 * j] = h->oeW[j];
+    t.count[2 * j] = (long long)oe_fan_in(h, j) * oe_fan_out(h, j); t.round[2 * j] = is_tc(h) ? 1 : 0;
+    t.src_off[2 * j + 1] = h->oe_var_off[2 * j + 1]; t.dst_off[2 * j + 1] = h->oeB[j];
+    t.count[2 * j + 1] = oe_fan_out(h, j); t.round[2 * j + 1] = 0;
+  }
+  // the workspace plan and the GEMM problem table grow by the encoder's buffers and problems
+  h->oe = true;
+  plan(h);
+  std::vector<DibGemmProblem> probs;
+  build_problems(h, probs);
+  h->h_probs = probs;
+  DibGemmProblem* dp = nullptr;
+  cudaError_t e = cudaMalloc(&dp, probs.size() * sizeof(DibGemmProblem));
+  if (e == cudaSuccess) e = cudaMemcpy(dp, probs.data(), probs.size() * sizeof(DibGemmProblem), cudaMemcpyHostToDevice);
+  if (e == cudaSuccess) e = cudaMalloc(&h->d_oe_col_src, col_src.size() * sizeof(int));
+  if (e == cudaSuccess) e = cudaMalloc(&h->d_oe_col_freq, col_freq.size() * sizeof(int));
+  if (e == cudaSuccess) e = cudaMemcpy(h->d_oe_col_src, col_src.data(), col_src.size() * sizeof(int), cudaMemcpyHostToDevice);
+  if (e == cudaSuccess) e = cudaMemcpy(h->d_oe_col_freq, col_freq.data(), col_freq.size() * sizeof(int), cudaMemcpyHostToDevice);
+  if (e != cudaSuccess) {
+    if (dp) cudaFree(dp);
+    return fail(std::string("dib_attach_output_encoder: CUDA error: ") + cudaGetErrorString(e));
+  }
+  cudaFree(h->d_probs);
+  h->d_probs = dp;
+  return 0;
+}
+
+int64_t dib_output_encoder_param_count(const dib_model* h) { return h && h->oe ? h->Q : -1; }
+
+int dib_output_encoder_param_layout(const dib_model* h, int64_t* offsets, int32_t* rows, int32_t* cols, int32_t capacity) {
+  if (!h || !h->oe) { fail("dib_output_encoder_param_layout: no output encoder attached"); return -1; }
+  const int nv = (int)h->oe_var_off.size();
+  if (!offsets || !rows || !cols) return nv;
+  if (capacity < nv) { fail("dib_output_encoder_param_layout: capacity too small"); return -1; }
+  for (int i = 0; i < nv; ++i) { offsets[i] = h->P + h->oe_var_off[i]; rows[i] = h->oe_var_rows[i]; cols[i] = h->oe_var_cols[i]; }
+  return nv;
+}
+
+int dib_output_encoder_forward(dib_model* h, const float* params, const float* y, int64_t n, float* out_e2, void* workspace,
+                               void* stream) {
+  if (check_call(h, params, y, n, workspace)) return 1;
+  if (!h->oe) return fail("dib_output_encoder_forward: no output encoder attached (dib_attach_output_encoder)");
+  if (!out_e2) return fail("dib_output_encoder_forward: null output");
+  if (n == 0) return 0;
+  Ctx c{h, params, static_cast<float*>(workspace), static_cast<cudaStream_t>(stream), (int)n};
+  if (oe_forward(c, y)) return 1;
+  DIB_CUDA_OK(dib_launch_copy2d(c.ws + h->oe_out.off, h->oe_out.ld, out_e2, h->out, h->out, n, c.st));
+  return 0;
+}
+
+int64_t dib_infonce_scratch_bytes(int32_t kind, int64_t n, int32_t d) {
+  if (kind == 0 || kind == 1 || kind == 4) return dib_infonce_head_tc_scratch_bytes(n, d);
+  if ((kind != 2 && kind != 3) || n < 1 || n > 32768 || d < 1 || d > 512) return -1;
+  return (n * n + 4 * n) * (int64_t)sizeof(float);
+}
+
+}  // extern "C"
+
+namespace {
+
+// dib_infonce_train_step (training) / dib_infonce_forward: model forward to e1 -> output encoder -> head -> external-loss
+// branch with y := d e1 -> [phased backward of the model -> output-encoder backward]
+int infonce_call(dib_model* h, const float* params, const float* x, const float* y, int64_t n, const float* beta_dev, int32_t kind,
+                 float temperature, const float* eps, uint64_t seed, uint32_t step, uint64_t sample_offset, void* head_scratch,
+                 float* grads_flat, float* out_stats, void* workspace, void* stream, bool training) {
+  const char* who = training ? "dib_infonce_train_step" : "dib_infonce_forward";
+  if (check_call(h, params, x, n, workspace)) return 1;
+  if (h->loss != DIB_LOSS_INFONCE || !h->oe)
+    return fail(std::string(who) + ": needs a DIB_LOSS_INFONCE handle with an attached output encoder");
+  if (!y || !beta_dev || !out_stats || !head_scratch || (training && !grads_flat))
+    return fail(std::string(who) + ": y, beta_dev, head_scratch, out_stats" + (training ? " and grads_flat" : "") + " are required");
+  if (n < 1) return fail(std::string(who) + ": the InfoNCE loss needs n >= 1 rows");
+  if (!(temperature > 0.f)) return fail(std::string(who) + ": temperature must be > 0");
+  const int D = h->out;
+  const bool gram = kind == 0 || kind == 1 || kind == 4;
+  if (gram) {
+    if (D > 256) return fail(std::string(who) + ": l2sq / l2 / cosine need output_dimensionality <= 256, got " + std::to_string(D));
+    if (reinterpret_cast<uintptr_t>(head_scratch) % 128) return fail(std::string(who) + ": head_scratch must be 128-byte aligned");
+    if (!dib_infonce_head_tc_available()) return fail(std::string(who) + ": cuTensorMapEncodeTiled is not available");
+  } else if (kind == 2 || kind == 3) {
+    if (n > 32768) return fail(std::string(who) + ": l1 / linf run the exact head, which holds n x n similarities: n <= 32768, got " +
+                               std::to_string(n));
+    if (D > 512) return fail(std::string(who) + ": l1 / linf need output_dimensionality <= 512");
+  } else {
+    return fail(std::string(who) + ": unknown similarity kind " + std::to_string(kind));
+  }
+  Ctx c{h, params, static_cast<float*>(workspace), static_cast<cudaStream_t>(stream), (int)n};
+  c.dev_step = training;
+  const float inv_batch = 1.f / (float)n;
+  int nblk_kl = 0;
+  if (run_forward(c, x, nullptr, eps, seed, step, sample_offset, inv_batch, training, nullptr, nullptr, out_stats, false, &nblk_kl))
+    return 1;
+  if (oe_forward(c, y)) return 1;
+  // the heads take unpadded [n, D] rows
+  float* cont = c.ws + h->oe_cont_off;
+  const long long nD = (long long)h->maxB * D;
+  float *e1 = c.ws + h->pred.off, *e2 = c.ws + h->oe_out.off, *de1 = cont + 2 * nD;
+  float* de2 = training ? c.ws + h->oe_dout.off : nullptr;
+  const bool padded = h->pred.ld != D;
+  if (padded) {
+    DIB_CUDA_OK(dib_launch_copy2d(e1, h->pred.ld, cont, D, D, n, c.st));
+    DIB_CUDA_OK(dib_launch_copy2d(e2, h->oe_out.ld, cont + nD, D, D, n, c.st));
+    e1 = cont; e2 = cont + nD;
+    if (training) de2 = cont + 3 * nD;
+  }
+  float* loss_dev = c.ws + h->nce_loss_off;
+  prof_begin(c, "infonce_head");
+  if (gram)
+    DIB_CUDA_OK(dib_launch_infonce_head_tc(kind, e1, e2, n, D, temperature, head_scratch, loss_dev, training ? de1 : nullptr, de2,
+                                           c.st));
+  else
+    DIB_CUDA_OK(dib_launch_infonce_head(kind, e1, e2, n, D, temperature, static_cast<float*>(head_scratch), loss_dev,
+                                        training ? de1 : nullptr, de2, c.st));
+  prof_end(c);
+  // d e2 into the output encoder's backward operand: rounded like d e1 (loss kernel) in the tensor-core modes, pads zeroed
+  if (training && (padded || is_tc(h)))
+    DIB_CUDA_OK(dib_launch_grad_handoff(de2, padded ? D : h->oe_dout.ld, c.ws + h->oe_dout.off, h->oe_dout.ld, D, n,
+                                        is_tc(h) ? 1 : 0, c.st));
+  if (loss_and_stats(c, training ? de1 : nullptr, inv_batch, training, nullptr, out_stats, nblk_kl)) return 1;
+  DIB_CUDA_OK(dib_launch_infonce_stats(loss_dev, n, out_stats + h->F, c.st));
+  if (!training) return 0;
+  if (train_phases(c, x, de1, n, beta_dev, inv_batch, eps, seed, step, sample_offset, grads_flat, out_stats, 3, true)) return 1;
+  long long rps = DIB_CEIL_DIV((long long)n, (long long)kMaxSplits);
+  if (rps < 256) rps = 256;
+  rps = DIB_ROUND_UP(rps, 64);
+  return oe_backward(c, (int)DIB_CEIL_DIV((long long)n, rps), (int)rps, grads_flat + h->P);
+}
+
+}  // namespace
+
+extern "C" {
+
+int dib_infonce_train_step(dib_model* h, const float* params, const float* x, const float* y, int64_t n, const float* beta_dev,
+                           int32_t kind, float temperature, const float* eps, uint64_t seed, uint32_t step,
+                           uint64_t sample_offset, void* head_scratch, float* grads_flat, float* out_stats, void* workspace,
+                           void* stream) {
+  return infonce_call(h, params, x, y, n, beta_dev, kind, temperature, eps, seed, step, sample_offset, head_scratch, grads_flat,
+                      out_stats, workspace, stream, true);
+}
+
+int dib_infonce_forward(dib_model* h, const float* params, const float* x, const float* y, int64_t n, const float* beta_dev,
+                        int32_t kind, float temperature, const float* eps, uint64_t seed, uint32_t step, uint64_t sample_offset,
+                        void* head_scratch, float* out_stats, void* workspace, void* stream) {
+  return infonce_call(h, params, x, y, n, beta_dev, kind, temperature, eps, seed, step, sample_offset, head_scratch, nullptr,
+                      out_stats, workspace, stream, false);
 }
 
 }  // extern "C"

@@ -96,6 +96,20 @@ bool dib_infonce_head_tc_available();
 cudaError_t dib_launch_infonce_head_tc(int kind, const float* e1, const float* e2, int64_t n, int d, float temperature,
                                        void* scratch, float* out_loss, float* d_e1, float* d_e2, cudaStream_t st);
 
+// InfoNCE train step (dib_infonce_train.cu): the output encoder's weight pack into its 16-byte-aligned shadow (variable v:
+// dst[dst_off[v] + i] = src[src_off[v] + i], TF32-rounded where round[v]), and stats[F] = n * L
+constexpr int kDibMaxOeLayers = 16;
+struct DibOePackTable {
+  int nvar = 0;
+  long long src_off[2 * (kDibMaxOeLayers + 1)], dst_off[2 * (kDibMaxOeLayers + 1)], count[2 * (kDibMaxOeLayers + 1)];
+  int round[2 * (kDibMaxOeLayers + 1)];
+};
+cudaError_t dib_launch_oe_pack(const float* src, float* dst, const DibOePackTable& t, cudaStream_t st);
+cudaError_t dib_launch_infonce_stats(const float* loss_dev, int64_t n, float* stats_loss, cudaStream_t st);
+// d e2 [n, cols] (row stride lds) -> dst rows of ldd floats: TF32-rounded when round_out, pad columns zeroed; src may be dst
+cudaError_t dib_launch_grad_handoff(const float* src, int lds, float* dst, int ldd, int cols, int64_t n, int round_out,
+                                    cudaStream_t st);
+
 cudaError_t dib_launch_metrics_update(const float* stats, const float* beta_dev, float* acc, int F, float kl_exponent,
                                       float kl_scale, cudaStream_t st);
 

@@ -90,10 +90,32 @@ class MeanSquaredError(_Loss):
         super().__init__(from_logits=True, name=name)
 
 
+class InfoNCE(_Loss):
+    """The InfoNCE training path of train.py:180-289 as a compiled loss: the model output e1 and a trainable output encoder's
+    e2 = output_encoder(y) (train.py:186-193) are compared with utils.get_scaled_similarity, and both networks are trained on
+    mean_i CE(i, S[i,:]) + mean_i CE(i, S^T[i,:]) + beta * sum_i KL_i (train.py:201-219).  Defaults are train.py:57-62's."""
+    kind = "infonce"
+
+    def __init__(self, similarity_type='l2', temperature=1.0, output_encoder_architecture=(128, 128), name=None):
+        from . import _lib
+        if similarity_type not in _lib.SIMILARITIES:
+            raise ValueError('Similarity type not implemented: ', similarity_type)          # utils.py:172
+        if not float(temperature) > 0.0:
+            raise ValueError(f"InfoNCE temperature must be > 0, got {temperature!r}")
+        arch = [int(w) for w in output_encoder_architecture]
+        if any(w < 1 for w in arch):
+            raise ValueError(f"output encoder widths must be >= 1, got {arch}")
+        super().__init__(from_logits=True, name=name)
+        self.similarity_type = similarity_type
+        self.temperature = float(temperature)
+        self.output_encoder_architecture = arch
+
+
 class losses:
     BinaryCrossentropy = BinaryCrossentropy
     SparseCategoricalCrossentropy = SparseCategoricalCrossentropy
     MeanSquaredError = MeanSquaredError
+    InfoNCE = InfoNCE
 
 
 def resolve_loss(loss):
@@ -114,6 +136,8 @@ def resolve_loss(loss):
             return "bce_probs"
         if key in ("external", "custom"):       # GradientTape-style loops: the caller owns the task loss
             return "external"
+        if key == "infonce":                    # dataset_dict['loss'] of the pendulum dataset (data.py:131)
+            return "infonce"
     raise ValueError(f"unsupported loss {loss!r}")
 
 

@@ -18,7 +18,7 @@ import torch
 
 from . import _lib
 from . import parallel
-from .keras_compat import Adam, RMSprop, SGD, Callback, History, optimizers, resolve_loss
+from .keras_compat import Adam, InfoNCE, RMSprop, SGD, Callback, History, optimizers, resolve_loss
 
 
 def _require_cuda():
@@ -230,6 +230,13 @@ class DistributedIBNet:
             self._lr_dev = torch.full((1,), 1e-3, dtype=torch.float32, device=self.device)
             self._step_dev = torch.zeros(1, dtype=torch.int32, device=self.device)
             self._epoch_acc = torch.zeros(self.number_features + 4, dtype=torch.float32, device=self.device)
+        # the optimizer updates [model P | output encoder Q] as ONE flat buffer (one Adam iteration count per step, train.py:219);
+        # without an output encoder these are the model's own buffers
+        self._params_all, self._m_all, self._v_all = self._params, self._m, self._v
+        self._Q = 0
+        self.output_encoder = None         # InfoNCE: built from the first y batch's width (build_output_encoder)
+        self._infonce = None               # the compiled keras_compat.InfoNCE
+        self._nce_scratch = {}             # (n, kind) -> head scratch of the InfoNCE step
         self._train_step_count = 0
         # ---- CUDA-graph replay of the train step (launch-bound small batches; fewer host calls per step at any size)
         env = os.environ.get("DIB_CUDA_GRAPH", "auto").lower()
@@ -295,8 +302,13 @@ class DistributedIBNet:
             finally:
                 self._lib.dib_destroy(h)
 
+    @property
+    def _PQ(self):
+        return self._P + self._Q
+
     def _ensure_handle(self, n):
-        key = (self._loss_kind, self.precision)
+        oe = self.output_encoder
+        key = (self._loss_kind, self.precision, None if oe is None else (oe.input_dimensionality, tuple(oe.architecture)))
         if self._handle is not None and self._handle_key == key and n <= self._max_batch:
             return
         self._release_handle()
@@ -306,6 +318,8 @@ class DistributedIBNet:
             cfg = self._config(max_batch)
             _lib.check(self._lib.dib_create(ctypes.byref(cfg), ctypes.byref(h)))
             self._handle, self._handle_key, self._max_batch = h, key, max_batch
+            if oe is not None and self._loss_kind == "infonce":
+                _lib.check(self._lib.dib_attach_output_encoder(h, ctypes.byref(oe._config())))
             self._graphs.clear(); self._graph_seen.clear()       # captured launches point into the old workspace
             self._step_dev_active = False
             if getattr(self, "_force_unfused", 0):
@@ -396,7 +410,96 @@ class DistributedIBNet:
         return t.contiguous()
 
     def _y_cols(self):
+        if self._loss_kind == "infonce":
+            if self.output_encoder is None:
+                raise RuntimeError("the InfoNCE output encoder is not built: pass a batch or call build_output_encoder(dy)")
+            return self.output_encoder.input_dimensionality
         return 0 if self._loss_kind == "sparse_ce_logits" else self.output_dimensionality
+
+    # ------------------------------------------------------------------ InfoNCE output encoder (train.py:186-193)
+    def build_output_encoder(self, input_dimensionality, architecture=None):
+        """Build the trainable output encoder y [n, input_dimensionality] -> e2 [n, output_dimensionality] of the InfoNCE
+        path (Keras builds it on its first call; fit / train_on_batch do this from the first y batch).  ``architecture``
+        defaults to the compiled InfoNCE loss's ``output_encoder_architecture``.  Weights: glorot-uniform kernels and zero
+        biases, drawn from a torch CPU generator seeded with ``seed + 0x5EED0E`` in flat order (a stream of its own, so the
+        model's initial weights do not depend on whether an output encoder exists)."""
+        if architecture is None:
+            architecture = self._infonce.output_encoder_architecture if self._infonce is not None else (128, 128)
+        dy, arch = int(input_dimensionality), [int(w) for w in architecture]
+        if self.output_encoder is not None:
+            if (self.output_encoder.input_dimensionality, self.output_encoder.architecture) == (dy, arch):
+                return self.output_encoder
+            raise ValueError("the output encoder is already built with a different shape")
+        oe = OutputEncoder(self, dy, arch)
+        with torch.cuda.device(self.device):
+            h = ctypes.c_void_p()
+            cfg = self._config(1)
+            cfg.loss, cfg.output_activation_fn = _lib.LOSSES["infonce"], 0
+            _lib.check(self._lib.dib_create(ctypes.byref(cfg), ctypes.byref(h)))
+            try:
+                _lib.check(self._lib.dib_attach_output_encoder(h, ctypes.byref(oe._config())))
+                Q = int(self._lib.dib_output_encoder_param_count(h))
+                nv = self._lib.dib_output_encoder_param_layout(h, None, None, None, 0)
+                offs, rows, cols = (ctypes.c_int64 * nv)(), (ctypes.c_int32 * nv)(), (ctypes.c_int32 * nv)()
+                assert self._lib.dib_output_encoder_param_layout(h, offs, rows, cols, nv) == nv
+            finally:
+                self._lib.dib_destroy(h)
+            oe._layout = (list(offs), list(rows), list(cols))
+            P = self._P
+            g = torch.Generator(device="cpu")
+            g.manual_seed(self.seed + 0x5EED0E)
+            q = torch.zeros(Q, dtype=torch.float32)
+            for off, r, c in zip(*oe._layout):
+                if r > 0:
+                    lim = math.sqrt(6.0 / (r + c))
+                    q[off - P:off - P + r * c] = (torch.rand(r * c, generator=g) * 2 - 1) * lim
+            self._release_handle()
+            self._graphs.clear(); self._graph_seen.clear()
+            new = []
+            for old, tail in ((self._params_all, q.to(self.device)), (self._m_all, None), (self._v_all, None)):
+                t = torch.zeros(P + Q, dtype=torch.float32, device=self.device)
+                t[:P].copy_(old[:P])
+                if tail is not None:
+                    t[P:].copy_(tail)
+                new.append(t)
+            self._params_all, self._m_all, self._v_all = new
+            self._params, self._m, self._v = (t[:P] for t in new)
+            self._Q = Q
+            self._gradstats = torch.zeros(P + Q + self.number_features + 3, dtype=torch.float32, device=self.device)
+        self.output_encoder = oe
+        return oe
+
+    def _head_scratch(self, n):
+        kind = _lib.SIMILARITIES[self._infonce.similarity_type]
+        t = self._nce_scratch.get((n, kind))
+        if t is None:
+            nbytes = int(self._lib.dib_infonce_scratch_bytes(kind, n, self.output_dimensionality))
+            # out of range (l1 / linf above 32768 rows): the step itself refuses with the reason
+            t = torch.empty(max(nbytes, 128), dtype=torch.uint8, device=self.device)
+            self._nce_scratch[(n, kind)] = t
+        return kind, t
+
+    def _infonce_call(self, x, y, step, sample_offset=0, eps=None, train=True, device_step=False, stats_out=None):
+        """dib_infonce_train_step (gradients into self._gradstats = [grads (P+Q) || stats]) or dib_infonce_forward."""
+        n = x.shape[0]
+        self._ensure_handle(n)
+        kind, scratch = self._head_scratch(n)
+        PQ = self._PQ
+        if train:
+            self._set_device_step(device_step)
+            _lib.check(self._lib.dib_infonce_train_step(
+                self._handle, _lib.ptr(self._params_all), _lib.ptr(x), _lib.ptr(y), n, _lib.ptr(self.beta._dev), kind,
+                self._infonce.temperature, _lib.ptr(eps), self.noise_seed, int(step) & 0xFFFFFFFF, int(sample_offset),
+                _lib.ptr(scratch), _lib.ptr(self._gradstats), _lib.ptr(self._gradstats[PQ:]), _lib.ptr(self._workspace),
+                _stream()))
+            return self._gradstats[PQ:]
+        stats = stats_out if stats_out is not None else torch.empty(self.number_features + 3, dtype=torch.float32,
+                                                                    device=self.device)
+        _lib.check(self._lib.dib_infonce_forward(
+            self._handle, _lib.ptr(self._params_all), _lib.ptr(x), _lib.ptr(y), n, _lib.ptr(self.beta._dev), kind,
+            self._infonce.temperature, _lib.ptr(eps), self.noise_seed, int(step) & 0xFFFFFFFF, int(sample_offset),
+            _lib.ptr(scratch), _lib.ptr(stats), _lib.ptr(self._workspace), _stream()))
+        return stats
 
     # ------------------------------------------------------------------ compute entry points
     def _forward(self, x, y, eps, step, sample_offset, want_pred=True, want_emb=False, stats_out=None):
@@ -467,6 +570,10 @@ class DistributedIBNet:
 
     def _backward(self, x, y, global_batch, eps=None, sample_offset=0, step=None, phases=3, device_step=False):
         """dib_train_step[_phased]: forward + reverse mode into self._gradstats = [grads (P) || stats (F+3)]."""
+        if self._loss_kind == "infonce":
+            st = 0 if device_step else (self._train_step_count if step is None else step)
+            self._infonce_call(x, y, st, sample_offset, eps, device_step=device_step)
+            return
         n = x.shape[0]
         self._ensure_handle(n)
         P = self._P
@@ -482,8 +589,8 @@ class DistributedIBNet:
         """optimizer.apply_gradients(zip(grads, model.trainable_variables)) of the custom loops (train.py:217-219,
         nb-bool cell 6): one Keras-Adam update of the flat parameter buffer with caller-supplied gradients."""
         g = torch.as_tensor(flat_grads, dtype=torch.float32).to(self.device).contiguous()
-        if g.numel() != self._P:
-            raise ValueError(f"expected {self._P} gradient values, got {g.numel()}")
+        if g.numel() != self._PQ:
+            raise ValueError(f"expected {self._PQ} gradient values, got {g.numel()}")
         self._sync_lr()
         with torch.cuda.device(self.device):
             self._optimizer_update(g)
@@ -496,12 +603,12 @@ class DistributedIBNet:
         opt = self.optimizer
         if isinstance(opt, Adam):
             _lib.check(self._lib.dib_adam_step(
-                _lib.ptr(self._params), _lib.ptr(grads), _lib.ptr(self._m), _lib.ptr(self._v), self._P,
+                _lib.ptr(self._params_all), _lib.ptr(grads), _lib.ptr(self._m_all), _lib.ptr(self._v_all), self._PQ,
                 _lib.ptr(self._lr_dev), _lib.ptr(self._step_dev), opt.beta_1, opt.beta_2, opt.epsilon, _stream()))
         else:
             h0, h1, h2 = opt.hyper()
             _lib.check(self._lib.dib_optimizer_step(
-                opt.kind, _lib.ptr(self._params), _lib.ptr(grads), _lib.ptr(self._m), _lib.ptr(self._v), self._P,
+                opt.kind, _lib.ptr(self._params_all), _lib.ptr(grads), _lib.ptr(self._m_all), _lib.ptr(self._v_all), self._PQ,
                 _lib.ptr(self._lr_dev), _lib.ptr(self._step_dev), h0, h1, h2, _stream()))
 
     def _adam(self):
@@ -528,7 +635,7 @@ class DistributedIBNet:
         """backward, all-reduce over the data-parallel group, Keras-Adam.  Replayed from CUDA graphs once a
         (batch size, offset) combination has run eagerly twice; the all-reduce is split into two buckets so that the
         first overlaps the encoder backward."""
-        P = self._P
+        P = self._PQ
         world, _ = parallel.world_and_rank(self.process_group)
         key = (int(x.shape[0]), int(global_batch), int(sample_offset), world)
         if self.use_cuda_graph and not self._graph_failed and eps is None and x.shape[0] > 0:
@@ -565,7 +672,7 @@ class DistributedIBNet:
                 self._ensure_handle(n)
                 self._set_device_step(True)
                 torch.cuda.synchronize(self.device)
-                keep = [t.clone() for t in (self._params, self._m, self._v, self._step_dev, self._noise_step_dev)]
+                keep = [t.clone() for t in (self._params_all, self._m_all, self._v_all, self._step_dev, self._noise_step_dev)]
                 graphs = []
                 launches0 = int(self._lib.dib_launch_count())
 
@@ -590,7 +697,7 @@ class DistributedIBNet:
                     cap(tail)
                 torch.cuda.synchronize(self.device)
                 # capture does not execute, but be safe against any eager side effect: restore the optimizer state
-                for t, k in zip((self._params, self._m, self._v, self._step_dev, self._noise_step_dev), keep):
+                for t, k in zip((self._params_all, self._m_all, self._v_all, self._step_dev, self._noise_step_dev), keep):
                     t.copy_(k)
         except Exception as e:       # noqa: BLE001 -- an unsupported capture falls back to eager launches, loudly
             import warnings
@@ -603,7 +710,7 @@ class DistributedIBNet:
         return g
 
     def _replay_step(self, g, x, y, world):
-        P = self._P
+        P = self._PQ
         if not self._step_dev_active or self._step_dev_dirty:
             self._set_device_step(True)
         self._replayed_launches += g["launches"]
@@ -629,7 +736,7 @@ class DistributedIBNet:
             yd = self._to_device(y, self._y_cols())
             e = self._to_device(eps) if eps is not None else None
             self._backward(xd, yd, global_batch or max(xd.shape[0], 1), e, sample_offset, step)
-            return self._gradstats[:self._P].clone(), self._gradstats[self._P:].clone()
+            return self._gradstats[:self._PQ].clone(), self._gradstats[self._PQ:].clone()
 
     # ------------------------------------------------------------------ encoder-only custom steps (SURVEY 8f3)
     def encode(self, x, eps=None, step=None, sample_offset=0):
@@ -726,10 +833,24 @@ class DistributedIBNet:
     def compile(self, optimizer='adam', loss=None, metrics=None, **_):
         """train.py:138-142."""
         new_opt = optimizers.get(optimizer)
+        kind = resolve_loss(loss)
+        if kind == "infonce":
+            nce = loss if isinstance(loss, InfoNCE) else InfoNCE()
+            self._check_infonce(nce, metrics)
+        elif self.output_encoder is not None:
+            # the optimizer buffers and gradient/statistics layout now span [model P | output encoder Q]
+            raise ValueError("this model has an InfoNCE output encoder: compile it with loss=InfoNCE")
+        old_nce = self._infonce
+        if kind == "infonce":
+            self._infonce = nce
+        # captured steps carry the loss (and the InfoNCE similarity / temperature) by value: re-capture after a change
+        sig = lambda c: None if c is None else (c.similarity_type, c.temperature)
+        if kind != self._loss_kind or (kind == "infonce" and sig(nce) != sig(old_nce)):
+            self._graphs.clear(); self._graph_seen.clear()
         if new_opt is not self.optimizer:        # a fresh Keras optimizer has fresh slots and iteration count
-            self._m.zero_(); self._v.zero_(); self._step_dev.zero_()
+            self._m_all.zero_(); self._v_all.zero_(); self._step_dev.zero_()
         self.optimizer = new_opt
-        self._loss_kind = resolve_loss(loss)
+        self._loss_kind = kind
         self.compiled_metrics_names = []
         for m in (metrics or []):
             if m not in ("accuracy", "acc"):
@@ -737,6 +858,22 @@ class DistributedIBNet:
             self.compiled_metrics_names.append("accuracy")
         self._lr_host = None
         self._sync_lr()
+
+    def _check_infonce(self, loss, metrics):
+        """compile(loss=InfoNCE(...)): what the InfoNCE step supports."""
+        if metrics:
+            raise ValueError(f"compile(loss=InfoNCE) takes no metrics (the InfoNCE path reports loss, KL{{i}} and beta), got {metrics!r}")
+        if self.output_activation_fn not in (None, "linear"):
+            raise ValueError("InfoNCE needs a linear output activation: the model output is the embedding e1 (train.py:117)")
+        if loss.similarity_type in ("l2sq", "l2", "cosine") and self.output_dimensionality > 256:
+            raise ValueError(f"InfoNCE with similarity {loss.similarity_type!r} needs output_dimensionality <= 256, "
+                             f"got {self.output_dimensionality}")
+        world, _ = parallel.world_and_rank(self.process_group)
+        if world > 1:
+            raise NotImplementedError("data-parallel InfoNCE training is not implemented: the loss couples every row of the "
+                                      "global batch")
+        if self.output_encoder is not None and self.output_encoder.architecture != loss.output_encoder_architecture:
+            raise ValueError("the output encoder is already built with a different architecture")
 
     def _sync_lr(self):
         """Device copy of optimizer.learning_rate (the step kernels read it from memory so that a schedule needs no re-capture);
@@ -760,6 +897,8 @@ class DistributedIBNet:
             D = sum(self.feature_dimensionalities)
             world, rank = parallel.world_and_rank(self.process_group)
             host_x = not (isinstance(x, torch.Tensor) and x.is_cuda)
+            if self._loss_kind == "infonce" and self.output_encoder is None:
+                self.build_output_encoder(int(np.shape(y)[-1]) if np.ndim(y) > 1 else 1)
             if sync or not host_x:
                 xd, yd = self._to_device(x, D), self._to_device(y, self._y_cols())
                 n = xd.shape[0]
@@ -824,6 +963,8 @@ class DistributedIBNet:
         if self.optimizer is None:
             raise RuntimeError("call compile() first")
         batch_size = 32 if batch_size is None else int(batch_size)
+        if self._loss_kind == "infonce":
+            return self._fit_infonce(x, y, batch_size, epochs, verbose, callbacks, validation_data, shuffle, initial_epoch)
         world, rank = parallel.world_and_rank(self.process_group)
         D = sum(self.feature_dimensionalities)
         with torch.cuda.device(self.device):
@@ -884,7 +1025,94 @@ class DistributedIBNet:
             self._metrics_update(stats)
         return self._read_epoch_logs(prefix="val_")
 
+    # ------------------------------------------------------------------ InfoNCE fit / evaluate (train.py:220-271)
+    def _fit_infonce(self, x, y, batch_size, epochs, verbose, callbacks, validation_data, shuffle, initial_epoch):
+        """fit for compile(loss=InfoNCE): full batches only.  Training step s reads rows [sB, (s+1)B) of the stream
+        perm_0 || perm_1 || ... (perm_k = epoch_permutation(k, N), or arange(N) with shuffle=False: train.py:224's repeated
+        dataset); epoch e runs steps [r(e), r(e+1)) with r(e) = np.round(e N / B) (train.py:236's epoch boundaries).  beta is
+        set by the callbacks' on_epoch_begin as in the Keras path -- train.py:241-250 changes it after the first step of an
+        epoch instead.  Validation: floor(Nv / B) + 1 full batches of consecutive rows of the repeated validation set
+        (train.py:230-234), noise keyed (2**31 + epoch, position in that stream).  Training noise: (optimizer step, row)."""
+        B = batch_size
+        with torch.cuda.device(self.device):
+            if self.output_encoder is None:
+                self.build_output_encoder(int(np.shape(y)[-1]) if np.ndim(y) > 1 else 1)
+            D = sum(self.feature_dimensionalities)
+            xd, yd = self._to_device(x, D), self._to_device(y, self._y_cols())
+            N = xd.shape[0]
+            if N < 1:
+                raise ValueError("fit needs at least one sample")
+            xv = yv = None
+            if validation_data is not None:
+                xv, yv = self._to_device(validation_data[0], D), self._to_device(validation_data[1], self._y_cols())
+            history = History()
+            cbs = list(callbacks or []) + [history]
+            for cb in cbs:
+                cb.set_model(self) if hasattr(cb, "set_model") else setattr(cb, "model", self)
+            self.history = history
+            self.stop_training = False
+            for cb in cbs:
+                getattr(cb, "on_train_begin", lambda logs=None: None)()
+            perms = {}
+
+            def stream_rows(s):
+                lo, hi = s * B, (s + 1) * B
+                parts = []
+                while lo < hi:
+                    k, r0 = divmod(lo, N)
+                    if k not in perms:
+                        perms[k] = self.epoch_permutation(k, N) if shuffle else torch.arange(N, device=self.device)
+                        for old in [j for j in perms if j < k - 1]:
+                            del perms[old]
+                    take = min(hi - lo, N - r0)
+                    parts.append(perms[k][r0:r0 + take])
+                    lo += take
+                return parts[0] if len(parts) == 1 else torch.cat(parts)
+
+            r = lambda e: int(np.round(e * N / B))
+            for epoch in range(initial_epoch, epochs):
+                for cb in cbs:
+                    cb.on_epoch_begin(epoch, logs=None)
+                self._sync_lr()
+                self._epoch_acc.zero_()
+                for s in range(r(epoch), r(epoch + 1)):
+                    idx = stream_rows(s)
+                    stats = self._train_step(xd.index_select(0, idx), yd.index_select(0, idx), global_batch=B)
+                    self._metrics_update(stats)
+                logs = self._read_epoch_logs()
+                if xv is not None:
+                    logs.update(self._evaluate_infonce(xv, yv, B, 2 ** 31 + epoch, prefix="val_"))
+                if verbose not in (False, 0):
+                    print(f"Epoch {epoch + 1}/{epochs} - " + " - ".join(
+                        f"{k}: {v:.4g}" for k, v in logs.items() if not k.removeprefix('val_').startswith('KL')))
+                for cb in cbs:
+                    cb.on_epoch_end(epoch, logs)
+                if self.stop_training:
+                    break
+            for cb in cbs:
+                getattr(cb, "on_train_end", lambda logs=None: None)()
+        return history
+
+    def _evaluate_infonce(self, xv, yv, B, step, prefix=""):
+        Nv = xv.shape[0]
+        self._epoch_acc.zero_()
+        stats = torch.empty(self.number_features + 3, dtype=torch.float32, device=self.device)
+        for b in range(Nv // B + 1):
+            idx = torch.arange(b * B, (b + 1) * B, device=self.device) % Nv
+            self._infonce_call(xv.index_select(0, idx), yv.index_select(0, idx), step, b * B, train=False, stats_out=stats)
+            self._metrics_update(stats)
+        return self._read_epoch_logs(prefix=prefix)
+
     def evaluate(self, x, y, batch_size=32, return_dict=True, **_):
+        if self._loss_kind == "infonce":
+            with torch.cuda.device(self.device):
+                if self.output_encoder is None:
+                    self.build_output_encoder(int(np.shape(y)[-1]) if np.ndim(y) > 1 else 1)
+                self._inference_calls += 1
+                D = sum(self.feature_dimensionalities)
+                logs = self._evaluate_infonce(self._to_device(x, D), self._to_device(y, self._y_cols()), int(batch_size),
+                                              (1 << 29) | (self._inference_calls & 0x1FFFFFFF))
+            return logs if return_dict else [logs["loss"]]
         with torch.cuda.device(self.device):
             world, rank = parallel.world_and_rank(self.process_group)
             D = sum(self.feature_dimensionalities)
@@ -924,7 +1152,9 @@ class PendingBatchResult:
             nn = max(s[F + 2], 1.0)
             m = self._m
             ib = self._beta * m.kl_loss_scale * (s[:F].sum() / nn) ** m.kl_loss_exponent      # models.py:118 / nb-chaos
-            out = {"loss": float(s[F] / nn + ib), "accuracy": float(s[F + 1] / nn)}
+            out = {"loss": float(s[F] / nn + ib)}
+            if m._loss_kind != "infonce":                     # the InfoNCE path has no accuracy
+                out["accuracy"] = float(s[F + 1] / nn)
             for i in range(F):
                 out[f"KL{i}"] = float(s[i] / nn)
             self._out = out
@@ -932,6 +1162,67 @@ class PendingBatchResult:
 
     def __getitem__(self, k):
         return self.get()[k]
+
+
+class OutputEncoder(_Network):
+    """model.output_encoder of the InfoNCE path (train.py:186-193): y [n, input_dimensionality] -> [PositionalEncoding] ->
+    Dense(w, activation_fn) per width -> Dense(output_dimensionality) -> e2.  Its variables are the [P, P+Q) tail of the
+    buffer the optimizer updates; ``model.trainable_variables`` / ``get_flat_weights`` stay the model's own."""
+
+    def __init__(self, model, input_dimensionality, architecture):
+        super().__init__(model, [])
+        self.input_dimensionality = int(input_dimensionality)
+        self.architecture = [int(w) for w in architecture]
+        self._layout = None
+
+    def _config(self):
+        self._c_arch = (ctypes.c_int32 * max(len(self.architecture), 1))(*self.architecture)
+        return _lib.DibOutputEncoderConfig(input_dimensionality=self.input_dimensionality, number_layers=len(self.architecture),
+                                           architecture=self._c_arch)
+
+    @property
+    def weights(self):
+        m = self._model
+        out = []
+        for off, r, c in zip(*self._layout):
+            v = m._params_all[off:off + max(r, 1) * c]
+            out.append(v.view(r, c) if r > 0 else v)
+        return out
+
+    trainable_variables = weights
+
+    def set_weights(self, weights):
+        vs = self.weights
+        if len(weights) != len(vs):
+            raise ValueError(f"expected {len(vs)} arrays, got {len(weights)}")
+        for v, w in zip(vs, weights):
+            v.copy_(torch.as_tensor(np.asarray(w), dtype=torch.float32).view(v.shape))
+
+    def get_flat_weights(self):
+        m = self._model
+        return m._params_all[m._P:].detach().cpu().numpy()
+
+    def set_flat_weights(self, flat):
+        m = self._model
+        m._params_all[m._P:].copy_(torch.as_tensor(np.asarray(flat), dtype=torch.float32))
+
+    def count_params(self):
+        return self._model._Q
+
+    def __call__(self, y, training=None):
+        m = self._model
+        with torch.cuda.device(m.device):
+            t = m._to_device(y, self.input_dimensionality)
+            n = t.shape[0]
+            if m._loss_kind != "infonce":
+                raise RuntimeError("the output encoder runs on a model compiled with loss=InfoNCE")
+            m._ensure_handle(max(n, 1))
+            out = torch.empty(n, m.output_dimensionality, dtype=torch.float32, device=m.device)
+            _lib.check(m._lib.dib_output_encoder_forward(m._handle, _lib.ptr(m._params_all), _lib.ptr(t), n, _lib.ptr(out),
+                                                         _lib.ptr(m._workspace), _stream()))
+        return _as_numpy_like(y, out)
+
+    call = __call__
 
 
 class InfoBottleneckAnnealingCallback(Callback):

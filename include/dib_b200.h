@@ -55,7 +55,12 @@ enum dib_loss {
   /* tf.keras.losses.BinaryCrossentropy() on PROBABILITIES (from_logits=False, the Keras default; use with
    * output_activation_fn = sigmoid): -[y log(p~ + eps) + (1-y) log(1 - p~ + eps)], p~ = clip(p, eps, 1-eps), eps = 1e-7
    * (keras.backend.binary_crossentropy); the gradient is zero where p is clipped. */
-  DIB_LOSS_BCE_PROBS = 4
+  DIB_LOSS_BCE_PROBS = 4,
+  /* the InfoNCE training path of train.py:180-289: the model output is the x-side embedding e1 (output_activation_fn must
+   * be linear; dib_forward with y = NULL returns e1).  A trainable output encoder (dib_attach_output_encoder) maps y to e2
+   * and dib_infonce_train_step trains both against the symmetric InfoNCE loss + beta * sum_i KL_i; dib_train_step refuses
+   * such a handle. */
+  DIB_LOSS_INFONCE = 5
 };
 
 /* arithmetic of the dense contractions; everything else (PE, exp, KL, loss, Adam, reductions) is fp32 in every mode
@@ -255,6 +260,48 @@ int dib_infonce_head(int32_t kind, const float* e1, const float* e2, int64_t n, 
 int64_t dib_infonce_head_tc_scratch_bytes(int64_t n, int32_t d);
 int dib_infonce_head_tc(int32_t kind, const float* e1, const float* e2, int64_t n, int32_t d, float temperature,
                         void* scratch, float* out_loss, float* d_e1, float* d_e2, void* stream);
+
+/* ---- InfoNCE training (train.py:180-289) on a DIB_LOSS_INFONCE handle ----------------------------------------------
+ * The output encoder of train.py:186-193: y [n, input_dimensionality] -> PositionalEncoding(2**arange(1, nfreq)) when the
+ * model uses it -> Dense(architecture[j], activation_fn) per width -> Dense(output_dimensionality) (linear), with the
+ * model's positional-encoding settings and activation.  Attach it once per handle, before the first call that uses it;
+ * dib_workspace_bytes then includes its buffers.  Its Q parameters follow the model's P ones: every call below takes
+ * params [P + Q], the encoder's variables in Keras order [W0, b0, W1, b1, ...] with [in, out] kernels at params[P, P+Q). */
+typedef struct dib_output_encoder_config {
+  int32_t input_dimensionality;      /* width of y */
+  int32_t number_layers;             /* len(infonce_y_encoder_architecture) (may be 0) */
+  const int32_t* architecture;       /* hidden widths */
+} dib_output_encoder_config;
+
+int dib_attach_output_encoder(dib_model* h, const dib_output_encoder_config* cfg);
+/* Q, or -1 (no encoder attached / null handle) */
+int64_t dib_output_encoder_param_count(const dib_model* h);
+/* as dib_param_layout; offsets index the [P + Q] buffer, so the first is P */
+int dib_output_encoder_param_layout(const dib_model* h, int64_t* offsets, int32_t* rows, int32_t* cols, int32_t capacity);
+/* output_encoder(y): y [n, input_dimensionality] -> out_e2 [n, output_dimensionality] */
+int dib_output_encoder_forward(dib_model* h, const float* params, const float* y, int64_t n, float* out_e2, void* workspace,
+                               void* stream);
+
+/* eval_batch_infonce(training=True) of train.py:201-219 minus the optimizer, with ONE model forward:
+ *   e1 = model(x) (noise as dib_train_step, including dib_set_noise_step_device), e2 = output_encoder(y),
+ *   L = mean_i CE(i, S[i,:]) + mean_i CE(i, S^T[i,:]) with S = get_scaled_similarity(e1, e2, kind, temperature),
+ *   loss = L + beta * sum_i KL_i.
+ * kind 0 'l2sq' | 1 'l2' | 4 'cosine' run the streaming tensor-core head (dib_infonce_head_tc: any n, output_dimensionality
+ * <= 256); 2 'l1' | 3 'linf' the exact head (n <= 32768).  head_scratch: dib_infonce_scratch_bytes(kind, n, D) bytes,
+ * 128-byte aligned.  grads_flat [P + Q] = d loss / d params, already batch-mean scaled; out_stats [F + 3] =
+ * [ sum_b KL_i (F) | n * L | 0 | n ], so dib_metrics_update_ex accumulates loss = L + IB term.  No allocation, no host
+ * synchronisation: CUDA-Graph capturable. */
+int dib_infonce_train_step(dib_model* h, const float* params, const float* x, const float* y, int64_t n, const float* beta_dev,
+                           int32_t kind, float temperature, const float* eps, uint64_t seed, uint32_t step,
+                           uint64_t sample_offset, void* head_scratch, float* grads_flat, float* out_stats, void* workspace,
+                           void* stream);
+/* the same without gradients: the validation pass (train.py:266); the by-value step is used, as in dib_forward */
+int dib_infonce_forward(dib_model* h, const float* params, const float* x, const float* y, int64_t n, const float* beta_dev,
+                        int32_t kind, float temperature, const float* eps, uint64_t seed, uint32_t step, uint64_t sample_offset,
+                        void* head_scratch, float* out_stats, void* workspace, void* stream);
+/* head_scratch bytes of the two calls above; -1 where they refuse (unknown kind, d > 256 for a Gram kind, n > 32768 for
+ * l1 / linf) */
+int64_t dib_infonce_scratch_bytes(int32_t kind, int64_t n, int32_t d);
 
 /* NEXT ROW f1 -- utils.estimate_mi_sandwich_bounds' per-batch kernel (utils.py:36-65): InfoNCE lower and leave-one-out
  * upper bound (nats) of I(U;X) for one encoder on one batch of n samples.  mu_logvar [n, 2E] (dib_encode_feature
